@@ -1,12 +1,16 @@
 #!/usr/bin/env python
 """Benchmark of the MIPSFusion per-frame neural-field hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Headline metric (BASELINE.json): map-step rays/s -- one mapping iteration = z-sampling, fused
 encode+MLP forward, SDF->weight render + losses, full backward, dense Adam -- on the BASELINE shape
 4096 rays x 43 samples, T = 2^19 hash grid, synthetic SDF-room frame.  The same JSON line also carries
 the tracking metric (pose candidates/s at 1024 x 2048) under "also".
+
+--dump-outputs DIR: after the K timed steps, writes what the last of them computed as DIR/<name>.npy (float32, see
+dump_outputs).  The inputs, the initial model and the device draws of the step are seeded, so two builds run with the same
+arguments can be compared output for output.
 
 N > 1 (torchrun): data-parallel mapping, one 4096-ray batch per rank (weak scaling), global mask counts
 all-reduced before the loss and gradients all-reduced before Adam (NCCL).
@@ -232,6 +236,10 @@ def run_gpu(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     dev_ms = float(t)
     value = world * R_RAYS * args.steps / (dev_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        sampler.pause()                 # (the copy and the file writes leave the GPU idle: kept out of the clock samples)
+        dump_outputs(args.dump_outputs, mapper, losses)
+        sampler.start()
 
     if args.quick:                    # profiling runs (ncu): only the timed steps above
         if rank == 0:
@@ -403,6 +411,24 @@ def run_gpu(args):
     if world > 1:
         import torch.distributed as dist
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, mapper, losses):
+    """Writes what the last timed map step computed, as float32 .npy files under out_dir (36 MB in all): the (8,) vector
+    FusedMapper.step returns, the rendered colour and depth of every ray, and the model the step leaves behind: the whole hash
+    grid (9,014,144 parameters) and the decoder's flat weights (36,577).
+    The backward accumulates the grid and decoder gradients with atomics in no fixed order, and Adam turns those last-bit
+    differences into whole steps wherever a gradient nearly cancels.  So two runs of one build do not agree bit for bit.
+    profiles/r3_dump_spread.txt records the per-array differences between two such runs (GPU, power limit and command included;
+    scripts/compare_dumps.py computes them).  They show the size of the spread from one pair of runs and are not a tolerance:
+    compare two builds against repeated runs of one of them."""
+    import numpy as np
+    import torch
+    b = mapper._bufs[(R_RAYS, S)]
+    arrays = {"losses": losses, "rgb": b["rgb"], "depth": b["depth"], "grid_params": mapper.grid, "decoder_params": mapper.mlp}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().to(torch.float32).cpu().numpy())
 
 
 def _max_over_ranks(x, dev, group):
@@ -934,7 +960,12 @@ if __name__ == "__main__":
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="timed steps only (for runs under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path (--impl b200)")
     if a.impl == "reference":
         run_reference(a)
     else:

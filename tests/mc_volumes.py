@@ -51,3 +51,13 @@ def cases():
     out["lattice_chains_eighths"] = (np.random.default_rng(9).integers(-2, 3, size=(18, 18, 18)).astype(np.float32) * 0.125,
                                      float(np.float32(0.125) - np.float32(1.1e-5)), 3.0)
     return out
+
+
+def fresh_cases():
+    """name -> (volume, isovalue, truncation): larger volumes than cases(), each at two levels (tests/golden/mcubes_fresh.npz)."""
+    rng = np.random.default_rng(123)
+    vols = {"sphere48": sphere((48, 40, 44), (23.1, 19.4, 22.2), 15.0, noise=0.3, seed=11),
+            "room56": room(56, seed=12),
+            "noise20": rng.standard_normal((20, 20, 20)).astype(np.float32) * 2.0,
+            "sphere40_scaled": sphere((40, 40, 40), (19.7, 20.2, 19.9), 14.0, noise=0.1, seed=13, scale=0.001)}
+    return {f"{name}_iso{k}": (vol, iso, 3.0) for name, vol in vols.items() for k, iso in enumerate((0.0, -0.21))}

@@ -45,19 +45,21 @@ def test_golden_volumes_are_the_seeded_ones(golden):
         assert np.array_equal(g[name + "_volume"], vol, equal_nan=True), name
 
 
-@pytest.mark.skipif(not omc.have_reference(), reason="oracle/_ref not built (needs /root/reference)")
-def test_oracle_matches_reference_binary_on_fresh_volumes():
-    """Fresh seeds, larger shapes: the restatement against the reference's own routine run here."""
+def test_oracle_matches_stored_outputs_on_fresh_volumes(golden):
+    """Fresh seeds, larger shapes (mc_volumes.fresh_cases()): the restatement against the stored outputs of
+    tests/golden/mcubes_fresh.npz, and against the reference's own routine as well where oracle/_ref has been built."""
+    import hashlib
     _ensure_oracle()
-    rng = np.random.default_rng(123)
-    vols = [mc_volumes.sphere((48, 40, 44), (23.1, 19.4, 22.2), 15.0, noise=0.3, seed=11),
-            mc_volumes.room(56, seed=12),
-            rng.standard_normal((20, 20, 20)).astype(np.float32) * 2.0,
-            mc_volumes.sphere((40, 40, 40), (19.7, 20.2, 19.9), 14.0, noise=0.1, seed=13, scale=0.001)]
-    for i, vol in enumerate(vols):
-        for iso in (0.0, -0.21):
-            a, b = omc.marching_cubes(vol, iso, 3.0), omc.reference_marching_cubes(vol, iso, 3.0)
-            assert _same(a, b), (i, iso)
+    g = golden("mcubes_fresh")
+    cases = mc_volumes.fresh_cases()
+    assert len(cases) == 8
+    for name, (vol, iso, trunc) in cases.items():
+        assert hashlib.sha256(np.ascontiguousarray(vol).tobytes()).hexdigest() == str(g[name + "_sha256"]), name
+        assert np.array_equal(g[name + "_args"], [iso, trunc]), name
+        a = omc.marching_cubes(vol, iso, trunc)
+        assert _same(a, (g[name + "_verts"].astype(np.float64), g[name + "_faces"].astype(np.uint64))), name
+        if omc.have_reference():
+            assert _same(a, omc.reference_marching_cubes(vol, iso, trunc)), name
 
 
 def test_oracle_input_dtypes_and_errors():
