@@ -306,6 +306,20 @@ int mf_pose_to_c2w(const float* state, float* c2w, void* stream);
 int mf_pose_refine_update(float* state, const float* c2w, const float* d_c2w, const float* losses, const float* loss_w,
                           double lr_rot, double lr_trans, int wait_iters, float* best_c2w, void* stream);
 
+/* ---- keyframe pose optimisation of the mapping loop (local_BA, mipsfusion.py:259-370: get_pose_param_optim :235-241,280-282,
+ * pose_optimizer.step() every pose_accum_step iterations :338-342) on the device, one thread per pose.  state (K x 24 floats):
+ * per pose [0:4] quaternion (w,x,y,z), [4:7] translation, [7:14] Adam m, [14:21] Adam v, [21] step count, [22:24] spare.
+ * frozen (K uint8, NULL = none frozen): poses that are not parameters (the submap's first keyframe; the current frame unless
+ * optim_cur); their poses_out entries are the input bit for bit and their state stays zero.
+ * mf_ba_pose_init: poses (K,4,4) -> quaternion (pytorch3d matrix_to_quaternion, standardised to a non-negative real part) and
+ * translation, zeroed moments and step; poses_out (K,4,4) = qt_to_transform_matrix of the parameters (geometry_helper.py:11-17). */
+int mf_ba_pose_init(const float* poses, const uint8_t* frozen, int K, float* state, float* poses_out, void* stream);
+/* One pose step: d_poses (K,4,4, rows 0-2 as mf_gen_rays_packed_bwd accumulates them) is pulled back to quaternion and
+ * translation, one torch.optim.Adam step (betas 0.9 / 0.999, eps 1e-8, lr_rot / lr_trans) is applied, poses_out is rebuilt and
+ * d_poses is zeroed (pose_optimizer.zero_grad()), frozen poses included. */
+int mf_ba_pose_update(float* state, float* d_poses, const uint8_t* frozen, int K, double lr_rot, double lr_trans,
+                      float* poses_out, void* stream);
+
 /* ---- a13: RandomOptimizer particle scoring (RandomOptimizer.py:54-73,81-85,113-131) ----
  * particles6 (C_total,6) pre-sampled template; search_size (6), rot_cur (3,3), trans_cur (3) device;
  * dirs_cam (P,3) and target_d (P) are the sampled pixels.  c_begin/c_count select this rank's candidate

@@ -12,6 +12,55 @@ __device__ __forceinline__ void quat_to_mat(const float q[4], float m[9]) {
     m[6] = two_s * (i * k - j * r); m[7] = two_s * (j * k + i * r); m[8] = 1 - two_s * (i * i + j * j);
 }
 
+// backward of qt_to_transform_matrix (geometry_helper.py:11-17): d_c2w (rows 0-2 of a row-major 4x4) -> g[7] =
+// d loss / d (quaternion, translation).  M = I + s * Q(q), s = 2 / |q|^2;  dM/dq_x = s * dQ/dq_x + Q * ds/dq_x, ds/dq_x = -s^2 q_x
+__device__ __forceinline__ void qt_backward(const float q[4], const float* __restrict__ d_c2w, float g[7]) {
+    const float r = q[0], i = q[1], j = q[2], k = q[3];
+    const float n2 = ((r * r + i * i) + j * j) + k * k, s = 2.0f / n2;
+    float G[9];
+    for (int a = 0; a < 3; ++a)
+        for (int b = 0; b < 3; ++b) G[a * 3 + b] = d_c2w[a * 4 + b];
+    const float Q[9] = {-(j * j + k * k), i * j - k * r, i * k + j * r, i * j + k * r, -(i * i + k * k), j * k - i * r,
+                        i * k - j * r, j * k + i * r, -(i * i + j * j)};
+    float gq_dot = 0.f;
+    for (int t = 0; t < 9; ++t) gq_dot += G[t] * Q[t];
+    const float dQr[9] = {0, -k, j, k, 0, -i, -j, i, 0};
+    const float dQi[9] = {0, j, k, j, -2 * i, -r, k, r, -2 * i};
+    const float dQj[9] = {-2 * j, i, r, i, 0, k, -r, k, -2 * j};
+    const float dQk[9] = {-2 * k, -r, i, r, -2 * k, j, i, j, 0};
+    g[0] = 0.f; g[1] = 0.f; g[2] = 0.f; g[3] = 0.f; g[4] = d_c2w[3]; g[5] = d_c2w[7]; g[6] = d_c2w[11];
+    for (int t = 0; t < 9; ++t) { g[0] += G[t] * dQr[t]; g[1] += G[t] * dQi[t]; g[2] += G[t] * dQj[t]; g[3] += G[t] * dQk[t]; }
+    const float qv[4] = {r, i, j, k};
+    for (int t = 0; t < 4; ++t) g[t] = s * g[t] - s * s * qv[t] * gq_dot;
+}
+
+// torch.optim.Adam (betas 0.9, 0.999, eps 1e-8, no weight decay) on the 7 pose parameters of a state laid out as
+// [0:4] quaternion, [4:7] translation, [7:14] m, [14:21] v, [21] step count; groups: quaternion lr_rot, translation lr_trans
+__device__ __forceinline__ void qt_adam_step(float* __restrict__ st, const float g[7], float lr_rot, float lr_trans) {
+    const float step = st[21] + 1.f;
+    st[21] = step;
+    const float bc1 = 1.f - powf(0.9f, step), bc2 = 1.f - powf(0.999f, step);
+    for (int t = 0; t < 7; ++t) {
+        float m = st[7 + t], v = st[14 + t];
+        m = 0.9f * m + 0.1f * g[t];
+        v = 0.999f * v + 0.001f * g[t] * g[t];
+        st[7 + t] = m; st[14 + t] = v;
+        const float lr = t < 4 ? lr_rot : lr_trans;
+        st[t] -= (lr / bc1) * m / (sqrtf(v) / sqrtf(bc2) + 1e-8f);
+    }
+}
+
+// c2w (row-major 4x4) = qt_to_transform_matrix(q, t)
+__device__ __forceinline__ void qt_to_c2w(const float q[4], const float t[3], float* __restrict__ c2w) {
+    float m[9];
+    quat_to_mat(q, m);
+    for (int r = 0; r < 3; ++r) {
+        for (int k = 0; k < 3; ++k) c2w[r * 4 + k] = m[r * 3 + k];
+        c2w[r * 4 + 3] = t[r];
+    }
+    c2w[12] = 0.f; c2w[13] = 0.f; c2w[14] = 0.f; c2w[15] = 1.f;
+}
+
 __device__ __forceinline__ void mat3_mul(const float a[9], const float b[9], float c[9]) {
 #pragma unroll
     for (int r = 0; r < 3; ++r)
@@ -300,13 +349,7 @@ MF_API int mf_ro_update_gathered(const float* gathered, int C, int per, double r
 // ---------------------------------------------------------------------------------------------
 __global__ void pose_to_c2w_kernel(const float* __restrict__ state, float* __restrict__ c2w) {
     if (threadIdx.x != 0) return;
-    float q[4] = {state[0], state[1], state[2], state[3]}, m[9];
-    quat_to_mat(q, m);                                                   // qt_to_transform_matrix, geometry_helper.py:11-17
-    for (int r = 0; r < 3; ++r) {
-        for (int k = 0; k < 3; ++k) c2w[r * 4 + k] = m[r * 3 + k];
-        c2w[r * 4 + 3] = state[4 + r];
-    }
-    c2w[12] = 0.f; c2w[13] = 0.f; c2w[14] = 0.f; c2w[15] = 1.f;
+    qt_to_c2w(state, state + 4, c2w);                                    // qt_to_transform_matrix, geometry_helper.py:11-17
 }
 
 __global__ void pose_refine_update_kernel(float* __restrict__ st, const float* __restrict__ c2w, const float* __restrict__ d_c2w,
@@ -332,37 +375,11 @@ __global__ void pose_refine_update_kernel(float* __restrict__ st, const float* _
         st[23] += 1.f;
     }
     if (st[23] > (float)wait_iters) { st[24] = 1.f; return; }            // break before backward / step
-    // ---- backward of qt_to_transform_matrix: d loss / d quaternion, d loss / d translation ----
-    const float r = st[0], i = st[1], j = st[2], k = st[3];
-    const float n2 = ((r * r + i * i) + j * j) + k * k, s = 2.0f / n2;
-    float G[9];
-    for (int a = 0; a < 3; ++a)
-        for (int b = 0; b < 3; ++b) G[a * 3 + b] = d_c2w[a * 4 + b];
-    // M = I + s * Q(q);  dM/dq_x = s * dQ/dq_x + Q * ds/dq_x,  ds/dq_x = -2 s q_x / n2 = -s^2 q_x
-    const float Q[9] = {-(j * j + k * k), i * j - k * r, i * k + j * r, i * j + k * r, -(i * i + k * k), j * k - i * r,
-                        i * k - j * r, j * k + i * r, -(i * i + j * j)};
-    float gq_dot = 0.f;
-    for (int t = 0; t < 9; ++t) gq_dot += G[t] * Q[t];
-    const float dQr[9] = {0, -k, j, k, 0, -i, -j, i, 0};
-    const float dQi[9] = {0, j, k, j, -2 * i, -r, k, r, -2 * i};
-    const float dQj[9] = {-2 * j, i, r, i, 0, k, -r, k, -2 * j};
-    const float dQk[9] = {-2 * k, -r, i, r, -2 * k, j, i, j, 0};
-    float g[7] = {0, 0, 0, 0, d_c2w[3], d_c2w[7], d_c2w[11]};
-    for (int t = 0; t < 9; ++t) { g[0] += G[t] * dQr[t]; g[1] += G[t] * dQi[t]; g[2] += G[t] * dQj[t]; g[3] += G[t] * dQk[t]; }
-    const float qv[4] = {r, i, j, k};
-    for (int t = 0; t < 4; ++t) g[t] = s * g[t] - s * s * qv[t] * gq_dot;
-    // ---- torch.optim.Adam (betas 0.9, 0.999, eps 1e-8, no weight decay), groups: quaternion lr_rot, translation lr_trans ----
-    const float step = st[21] + 1.f;
-    st[21] = step;
-    const float bc1 = 1.f - powf(0.9f, step), bc2 = 1.f - powf(0.999f, step);
-    for (int t = 0; t < 7; ++t) {
-        float m = st[7 + t], v = st[14 + t];
-        m = 0.9f * m + 0.1f * g[t];
-        v = 0.999f * v + 0.001f * g[t] * g[t];
-        st[7 + t] = m; st[14 + t] = v;
-        const float lr = t < 4 ? lr_rot : lr_trans;
-        st[t] -= (lr / bc1) * m / (sqrtf(v) / sqrtf(bc2) + 1e-8f);
-    }
+    // ---- backward of qt_to_transform_matrix, then one torch.optim.Adam step with the groups quaternion / translation ----
+    const float q[4] = {st[0], st[1], st[2], st[3]};
+    float g[7];
+    qt_backward(q, d_c2w, g);
+    qt_adam_step(st, g, lr_rot, lr_trans);
 }
 
 MF_API int mf_pose_to_c2w(const float* state, float* c2w, void* stream) {
@@ -377,6 +394,87 @@ MF_API int mf_pose_refine_update(float* state, const float* c2w, const float* d_
     MF_CHECK_ARG(state && c2w && d_c2w && losses && loss_w && best_c2w);
     pose_refine_update_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(state, c2w, d_c2w, losses, loss_w, (float)lr_rot, (float)lr_trans,
                                                                  wait_iters, best_c2w);
+    MF_LAUNCH_CHECK();
+    return MF_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Keyframe pose optimisation of the mapping loop (local_BA, mipsfusion.py:259-370; get_pose_param_optim :235-241,280-282;
+// pose step :338-342): K pose states of BA_STATE floats, one thread per pose.
+// ---------------------------------------------------------------------------------------------
+constexpr int BA_STATE = 24;
+
+// pytorch3d matrix_to_quaternion (rotation_conversions.py) for one row-major 3x3 block of a 4x4, in the op order of the
+// torch formula (tracker.matrix_to_quaternion): real part first, standardised to a non-negative real part
+__device__ __forceinline__ void mat_to_quat(const float* __restrict__ P, float q[4]) {
+    const float m00 = P[0], m01 = P[1], m02 = P[2], m10 = P[4], m11 = P[5], m12 = P[6], m20 = P[8], m21 = P[9], m22 = P[10];
+    const float qa[4] = {__fadd_rn(__fadd_rn(__fadd_rn(1.0f, m00), m11), m22), __fsub_rn(__fsub_rn(__fadd_rn(1.0f, m00), m11), m22),
+                         __fsub_rn(__fadd_rn(__fsub_rn(1.0f, m00), m11), m22), __fadd_rn(__fsub_rn(__fsub_rn(1.0f, m00), m11), m22)};
+    float q_abs[4];
+    for (int a = 0; a < 4; ++a) q_abs[a] = qa[a] > 0.f ? __fsqrt_rn(qa[a]) : 0.f;
+    int best = 0;                                                        // torch.argmax: the first of equal maxima
+    for (int a = 1; a < 4; ++a)
+        if (q_abs[a] > q_abs[best]) best = a;
+    float c[4];
+    const float sq = __fmul_rn(q_abs[best], q_abs[best]);
+    switch (best) {
+        case 0: c[0] = sq; c[1] = __fsub_rn(m21, m12); c[2] = __fsub_rn(m02, m20); c[3] = __fsub_rn(m10, m01); break;
+        case 1: c[0] = __fsub_rn(m21, m12); c[1] = sq; c[2] = __fadd_rn(m10, m01); c[3] = __fadd_rn(m02, m20); break;
+        case 2: c[0] = __fsub_rn(m02, m20); c[1] = __fadd_rn(m10, m01); c[2] = sq; c[3] = __fadd_rn(m12, m21); break;
+        default: c[0] = __fsub_rn(m10, m01); c[1] = __fadd_rn(m20, m02); c[2] = __fadd_rn(m21, m12); c[3] = sq; break;
+    }
+    const float den = __fmul_rn(2.0f, fmaxf(q_abs[best], 0.1f));
+    for (int a = 0; a < 4; ++a) q[a] = __fdiv_rn(c[a], den);
+    if (q[0] < 0.f)
+        for (int a = 0; a < 4; ++a) q[a] = -q[a];
+}
+
+__global__ void ba_pose_init_kernel(const float* __restrict__ poses, const uint8_t* __restrict__ frozen, int K,
+                                    float* __restrict__ state, float* __restrict__ poses_out) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= K) return;
+    const float* P = poses + k * 16;
+    float* s = state + k * BA_STATE;
+    for (int t = 0; t < BA_STATE; ++t) s[t] = 0.f;
+    if (frozen && frozen[k]) {                                           // not a parameter: copied through bit for bit
+        for (int t = 0; t < 16; ++t) poses_out[k * 16 + t] = P[t];
+        return;
+    }
+    float q[4];
+    mat_to_quat(P, q);
+    for (int t = 0; t < 4; ++t) s[t] = q[t];
+    s[4] = P[3]; s[5] = P[7]; s[6] = P[11];
+    qt_to_c2w(s, s + 4, poses_out + k * 16);                             // poses_all is built from the parameters (:280-282)
+}
+
+__global__ void ba_pose_update_kernel(float* __restrict__ state, float* __restrict__ d_poses, const uint8_t* __restrict__ frozen,
+                                      int K, float lr_rot, float lr_trans, float* __restrict__ poses_out) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= K) return;
+    float* dP = d_poses + k * 16;
+    if (!(frozen && frozen[k])) {
+        float* s = state + k * BA_STATE;
+        const float q[4] = {s[0], s[1], s[2], s[3]};
+        float g[7];
+        qt_backward(q, dP, g);
+        qt_adam_step(s, g, lr_rot, lr_trans);
+        qt_to_c2w(s, s + 4, poses_out + k * 16);
+    }
+    for (int t = 0; t < 16; ++t) dP[t] = 0.f;                            // pose_optimizer.zero_grad() after the step (:338-342)
+}
+
+MF_API int mf_ba_pose_init(const float* poses, const uint8_t* frozen, int K, float* state, float* poses_out, void* stream) {
+    MF_CHECK_ARG(poses && state && poses_out && K > 0);
+    ba_pose_init_kernel<<<(K + 63) / 64, 64, 0, (cudaStream_t)stream>>>(poses, frozen, K, state, poses_out);
+    MF_LAUNCH_CHECK();
+    return MF_OK;
+}
+
+MF_API int mf_ba_pose_update(float* state, float* d_poses, const uint8_t* frozen, int K, double lr_rot, double lr_trans,
+                             float* poses_out, void* stream) {
+    MF_CHECK_ARG(state && d_poses && poses_out && K > 0);
+    ba_pose_update_kernel<<<(K + 63) / 64, 64, 0, (cudaStream_t)stream>>>(state, d_poses, frozen, K, (float)lr_rot, (float)lr_trans,
+                                                                       poses_out);
     MF_LAUNCH_CHECK();
     return MF_OK;
 }

@@ -81,11 +81,12 @@ class KeyframeRayStore:
         return first, pix_num - first - last, last
 
     def sample_rays_in_submap(self, first_kf_Id, related_kf_ids, pix_num, idx_first=None, idx_other=None, idx_last=None,
-                              seed=None, out=None, return_draws=False):
+                              seed=None, out=None, return_draws=False, out_ids=None):
         """-> sampled_rays (n,7), kf_ids (n,), kf_indices (n,) on the device, in the reference's order (first keyframe,
         other related keyframes, latest keyframe).  idx_* : explicit index draws (int64); without them the draws are
         made inside the gather kernel (one launch; ``seed`` fixes them, ``return_draws`` also returns the indices).
-        ``out``: optional (>= n, 7) device buffer that receives the rays."""
+        ``out``: optional (>= n, 7) device buffer that receives the rays; ``out_ids``: optional pair of (n,) int64 device
+        buffers that receive kf_ids and kf_indices (device draws only)."""
         dev = self.device
         related = torch.as_tensor(related_kf_ids, dtype=torch.int64).reshape(-1)
         n_rel = int(related.shape[0])
@@ -95,7 +96,10 @@ class KeyframeRayStore:
         if idx_first is None and idx_other is None and idx_last is None:
             n = n_first + n_other + n_last
             rays = torch.empty(n, 7, device=dev, dtype=torch.float32) if out is None else out[:n]
-            kf_ids = torch.empty(n, device=dev, dtype=torch.int64); kf_indices = torch.empty_like(kf_ids)
+            if out_ids is None:
+                kf_ids = torch.empty(n, device=dev, dtype=torch.int64); kf_indices = torch.empty_like(kf_ids)
+            else:
+                kf_ids, kf_indices = out_ids
             draws = torch.empty(n, device=dev, dtype=torch.int64) if return_draws else None
             key = tuple(int(v) for v in other_ids)
             cache = self.__dict__.setdefault("_ids_cache", {})

@@ -14,6 +14,7 @@ import torch
 from . import _lib as L
 from . import dist as D
 from .decoder import _Workspace
+from .keyframe_store import _new_seed
 
 
 class FusedMapper:
@@ -202,54 +203,150 @@ class FusedMapper:
         hb["rays7"].copy_(rays7, non_blocking=True)
         if pose_idx is not None:
             hb["idx"].copy_(pose_idx, non_blocking=True)
-        poses = poses.contiguous()
-        L.call("mf_gen_rays_packed", L.ptr(hb["rays7"]), L.ptr(poses), L.ptr(hb["idx"]) if pose_idx is not None else None,
-               L.ptr(hb["o"]), L.ptr(hb["d"]), L.ptr(hb["rgb"]), L.ptr(hb["depth"]), R, poses.shape[0], L.stream())
-        self.launches += 1
-        if not pose_grad:
-            losses = self.step(hb["o"], hb["d"], hb["rgb"], hb["depth"], EMD_w=EMD_w)
-            hb["out"].copy_(losses, non_blocking=True)
-            torch.cuda.current_stream(self.dev).synchronize()
-            return hb["out"]
-        if "d_o" not in hb:
-            hb["d_o"], hb["d_d"] = torch.empty_like(hb["o"]), torch.empty_like(hb["d"])
-        losses = self.step(hb["o"], hb["d"], hb["rgb"], hb["depth"], EMD_w=EMD_w, ray_grads=(hb["d_o"], hb["d_d"]))
-        d_poses = torch.zeros(poses.shape[0], 4, 4, device=self.dev, dtype=torch.float32)
-        L.call("mf_gen_rays_packed_bwd", L.ptr(hb["rays7"]), L.ptr(hb["idx"]) if pose_idx is not None else None, L.ptr(hb["d_o"]),
-               L.ptr(hb["d_d"]), L.ptr(d_poses), R, poses.shape[0], L.stream())
-        self.launches += 2
-        if self.world > 1:                                           # every rank holds the same poses: sum the gradients
-            D.allreduce_sum_(d_poses, self.group)
-            d_poses.mul_(1.0 / self.world)
+        res = self._step_packed(hb, hb["idx"] if pose_idx is not None else None, poses, EMD_w, pose_grad)
+        losses = res[0] if pose_grad else res
         hb["out"].copy_(losses, non_blocking=True)
         torch.cuda.current_stream(self.dev).synchronize()
-        return hb["out"], d_poses
+        return (hb["out"], res[1]) if pose_grad else hb["out"]
 
-    def step_from_store(self, store, first_kf_Id, related_kf_ids, poses_all, pix_num, cur_rays7=None, EMD_w=0.01, **draws):
-        """One mapping iteration fed from the device-resident keyframe ray store (steps 3.1-3.4 of the reference's BA
-        loop, mipsfusion.py:293-335, without any host data): sample ``pix_num`` rays of the submap's keyframes
-        (:class:`KeyframeRayStore.sample_rays_in_submap`), append the current frame's rays ``cur_rays7`` (n,7; pose index
-        -1 = last pose), generate the rays with ``poses_all`` (K,4,4) and run :meth:`step`.  Returns the device losses."""
+    def _step_packed(self, b, pose_idx, poses, EMD_w, pose_grad, u=None, d_poses=None):
+        """The mapping iteration on a packed batch already on the device (``b["rays7"]`` (R,7), ``pose_idx`` (R,) or None):
+        ray generation with ``poses`` (K,4,4), :meth:`step`, and with ``pose_grad`` the pose-gradient leg.  Returns the device
+        losses, with ``pose_grad`` (losses, d_poses): ``d_poses`` (K,4,4) is ADDED to when given (the BA loop's accumulation
+        across iterations), else a fresh zeroed tensor that is averaged over the ranks before it is returned."""
+        R = b["rays7"].shape[0]
+        poses = poses if (poses.is_cuda and poses.dtype == torch.float32 and poses.is_contiguous()) \
+            else poses.to(self.dev, torch.float32).contiguous()
+        K = poses.shape[0]
+        L.call("mf_gen_rays_packed", L.ptr(b["rays7"]), L.ptr(poses), L.ptr(pose_idx), L.ptr(b["o"]), L.ptr(b["d"]), L.ptr(b["rgb"]),
+               L.ptr(b["depth"]), R, K, L.stream())
+        self.launches += 1
+        if not pose_grad:
+            return self.step(b["o"], b["d"], b["rgb"], b["depth"], u=u, EMD_w=EMD_w)
+        if "d_o" not in b:
+            b["d_o"], b["d_d"] = torch.empty_like(b["o"]), torch.empty_like(b["d"])
+        losses = self.step(b["o"], b["d"], b["rgb"], b["depth"], u=u, EMD_w=EMD_w, ray_grads=(b["d_o"], b["d_d"]))
+        average = d_poses is None
+        if average:
+            d_poses = torch.zeros(K, 4, 4, device=self.dev, dtype=torch.float32)
+            self.launches += 1
+        L.call("mf_gen_rays_packed_bwd", L.ptr(b["rays7"]), L.ptr(pose_idx), L.ptr(b["d_o"]), L.ptr(b["d_d"]), L.ptr(d_poses), R, K,
+               L.stream())
+        self.launches += 1
+        if average:
+            self._average_pose_grads(d_poses)
+        return losses, d_poses
+
+    def _average_pose_grads(self, d_poses):
+        if self.world > 1:                                           # every rank holds the same poses: average the gradients
+            D.allreduce_sum_(d_poses, self.group)
+            d_poses.mul_(1.0 / self.world)
+
+    def _store_batch(self, store, first_kf_Id, related_kf_ids, pix_num, cur_rays7, **draws):
+        """Packed batch buffers of (pix_num, n_cur) filled from the keyframe ray store: ``pix_num`` rays of the submap's
+        keyframes (:meth:`KeyframeRayStore.sample_rays_in_submap`, pose index = slot in ``related_kf_ids``), then the current
+        frame's rays ``cur_rays7`` (pose index -1 = last pose)."""
         n_cur = 0 if cur_rays7 is None else int(cur_rays7.shape[0])
-        R = int(pix_num) + n_cur
-        sb = self._bufs.get(("store", int(pix_num), n_cur))       # (keyed by the split: the tail of `idx` must stay -1)
+        pix_num = int(pix_num)
+        R = pix_num + n_cur
+        sb = self._bufs.get(("store", pix_num, n_cur))             # (keyed by the split: the tail of `idx` must stay -1)
         if sb is None:
             f32 = dict(device=self.dev, dtype=torch.float32)
             sb = dict(rays7=torch.empty(R, 7, **f32), idx=torch.full((R,), -1, device=self.dev, dtype=torch.int64),
+                      kf_ids=torch.empty(pix_num, device=self.dev, dtype=torch.int64),
                       o=torch.empty(R, 3, **f32), d=torch.empty(R, 3, **f32), rgb=torch.empty(R, 3, **f32), depth=torch.empty(R, **f32))
-            self._bufs[("store", int(pix_num), n_cur)] = sb
-        rays, _, kf_indices = store.sample_rays_in_submap(first_kf_Id, related_kf_ids, pix_num, out=sb["rays7"], **draws)[:3]
-        if rays.data_ptr() != sb["rays7"].data_ptr():               # explicit draws: gathered into a fresh tensor
-            sb["rays7"][:pix_num].copy_(rays)
-        sb["idx"][:pix_num].copy_(kf_indices)                       # the tail stays -1: current frame = last pose
+            self._bufs[("store", pix_num, n_cur)] = sb
+        if any(draws.get(k) is not None for k in ("idx_first", "idx_other", "idx_last")):
+            rays, _, kf_indices = store.sample_rays_in_submap(first_kf_Id, related_kf_ids, pix_num, **draws)[:3]
+            sb["rays7"][:pix_num].copy_(rays)                       # explicit draws: gathered into a fresh tensor
+            sb["idx"][:pix_num].copy_(kf_indices)
+        else:                                                       # device draws: the gather writes straight into the batch
+            store.sample_rays_in_submap(first_kf_Id, related_kf_ids, pix_num, out=sb["rays7"],
+                                        out_ids=(sb["kf_ids"], sb["idx"][:pix_num]), **draws)
         if n_cur:
             sb["rays7"][pix_num:].copy_(cur_rays7)
-        poses = poses_all if (poses_all.is_cuda and poses_all.dtype == torch.float32 and poses_all.is_contiguous()) \
+        self.launches += 1
+        return sb
+
+    def step_from_store(self, store, first_kf_Id, related_kf_ids, poses_all, pix_num, cur_rays7=None, EMD_w=0.01, pose_grad=False,
+                        **draws):
+        """One mapping iteration fed from the device-resident keyframe ray store (steps 3.1-3.4 of the reference's BA
+        loop, mipsfusion.py:293-335, without any host data): sample ``pix_num`` rays of the submap's keyframes
+        (:class:`KeyframeRayStore.sample_rays_in_submap`), append the current frame's rays ``cur_rays7`` (n,7; pose index
+        -1 = last pose), generate the rays with ``poses_all`` (K,4,4) and run :meth:`step`.  Returns the device losses;
+        pose_grad=True returns (losses, d_poses) with d_poses as :meth:`step_host` returns it (rank average included)."""
+        sb = self._store_batch(store, first_kf_Id, related_kf_ids, pix_num, cur_rays7, **draws)
+        return self._step_packed(sb, sb["idx"], poses_all, EMD_w, pose_grad)
+
+    def local_ba(self, store, first_kf_Id, related_kf_ids, poses_all, pix_num, cur_rays7=None, n_iters=None, pose_accum_step=None,
+                 lr_rot=None, lr_trans=None, optim_cur=None, seed=None, u=None, EMD_w=0.01):
+        """The reference's local bundle adjustment (MIPSFusion.local_BA, mipsfusion.py:259-370; the same body runs in
+        InactiveMap.local_BA, local_BA_switch and initialize_new_localMLP) on the device: ``n_iters`` mapping iterations fed from
+        the keyframe ray store (as :meth:`step_from_store`) that also accumulate d loss / d poses, and every ``pose_accum_step``
+        iterations one Adam step on the keyframe poses (quaternion + translation, get_pose_param_optim :235-241,280-282,
+        step :338-342).  Gradients of a trailing partial period are dropped, as in the reference.
+
+        poses_all (K,4,4): the related keyframes' poses in the order of ``related_kf_ids``, then the current frame's.  Pose 0
+        (the submap's first keyframe) is never optimised, the last one only with ``optim_cur``; both come back bit for bit.
+        n_iters, pose_accum_step, lr_rot, lr_trans, optim_cur: ``config["mapping"]`` keys iters, pose_accum_step, lr_rot,
+        lr_trans, optim_cur unless given.  seed: base of the ray draws (rank r, iteration i draw with seed + 3 (i world + r),
+        the three segment seeds of mf_kf_sample_rays); from torch's CPU generator when None.  u: optional (n_iters, R, S)
+        stratified jitter.  With a process group every rank draws its own rays and the pose gradients are averaged over the
+        ranks once per pose step, so all ranks hold the same poses.
+
+        -> (poses (K,4,4), losses (n_iters, 8)) device tensors, overwritten by the next call of the same shape.  No host
+        synchronisation; no allocation after the first call for a (K, pix_num, n_cur, n_iters)."""
+        mc = self.model.config.get("mapping", {})
+
+        def hp(v, key):
+            if v is not None:
+                return v
+            if key not in mc:
+                raise L.MipsFusionB200Error("local_ba: %s not given and config['mapping'] has no '%s'" % (key, key))
+            return mc[key]
+        n_iters, accum = int(hp(n_iters, "iters")), int(hp(pose_accum_step, "pose_accum_step"))
+        lr_rot, lr_trans, optim_cur = float(hp(lr_rot, "lr_rot")), float(hp(lr_trans, "lr_trans")), bool(hp(optim_cur, "optim_cur"))
+        if accum < 1:
+            raise L.MipsFusionB200Error("local_ba: pose_accum_step must be >= 1")
+        self.model.decoder.prepared()                                # adopt external writes to the decoder's parameters
+        K = int(poses_all.shape[0])
+        n_cur = 0 if cur_rays7 is None else int(cur_rays7.shape[0])
+        key = ("ba", K, int(pix_num), n_cur)
+        bb = self._bufs.get(key)
+        if bb is None:
+            f32 = dict(device=self.dev, dtype=torch.float32)
+            bb = self._bufs[key] = dict(state=torch.zeros(K, 24, **f32), poses=torch.empty(K, 4, 4, **f32),
+                                        d_poses=torch.zeros(K, 4, 4, **f32), frozen={}, losses={})
+        frozen = bb["frozen"].get(optim_cur)
+        if frozen is None:
+            f = torch.zeros(K, dtype=torch.uint8)
+            f[0] = 1                                                 # get_pose_param_optim(poses[1:])
+            if not optim_cur:
+                f[-1] = 1
+            frozen = bb["frozen"][optim_cur] = f.to(self.dev)
+        losses = bb["losses"].get(n_iters)
+        if losses is None:
+            losses = bb["losses"][n_iters] = torch.zeros(n_iters, 8, device=self.dev, dtype=torch.float32)
+        poses_in = poses_all if (poses_all.is_cuda and poses_all.dtype == torch.float32 and poses_all.is_contiguous()) \
             else poses_all.to(self.dev, torch.float32).contiguous()
-        L.call("mf_gen_rays_packed", L.ptr(sb["rays7"]), L.ptr(poses), L.ptr(sb["idx"]), L.ptr(sb["o"]), L.ptr(sb["d"]), L.ptr(sb["rgb"]),
-               L.ptr(sb["depth"]), R, poses.shape[0], L.stream())
+        st = L.stream()
+        L.call("mf_ba_pose_init", L.ptr(poses_in), L.ptr(frozen), K, L.ptr(bb["state"]), L.ptr(bb["poses"]), st)
+        bb["d_poses"].zero_()
         self.launches += 2
-        return self.step(sb["o"], sb["d"], sb["rgb"], sb["depth"], EMD_w=EMD_w)
+        seed = _new_seed() if seed is None else int(seed)
+        world, rank = D.world(self.group)
+        for i in range(n_iters):
+            sb = self._store_batch(store, first_kf_Id, related_kf_ids, pix_num, cur_rays7, seed=(seed + 3 * (i * world + rank)) & 0xffffffff)
+            li, _ = self._step_packed(sb, sb["idx"], bb["poses"], EMD_w, True, u=None if u is None else L.f32c(u[i], self.dev),
+                                      d_poses=bb["d_poses"])
+            losses[i].copy_(li)
+            self.launches += 1
+            if (i + 1) % accum == 0:
+                self._average_pose_grads(bb["d_poses"])
+                L.call("mf_ba_pose_update", L.ptr(bb["state"]), L.ptr(bb["d_poses"]), L.ptr(frozen), K, lr_rot, lr_trans,
+                       L.ptr(bb["poses"]), st)
+                self.launches += 1
+        return bb["poses"], losses
 
     def apply_gradients(self):
         """Adam on (grid, decoder) with the reference's groups (mipsfusion.py:580-584), zero_grad fused in."""
