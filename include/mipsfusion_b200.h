@@ -305,6 +305,11 @@ int mf_pose_to_c2w(const float* state, float* c2w, void* stream);
  * quaternion and the translation and one torch.optim.Adam step (betas 0.9 / 0.999, eps 1e-8) with lr_rot / lr_trans is applied. */
 int mf_pose_refine_update(float* state, const float* c2w, const float* d_c2w, const float* losses, const float* loss_w,
                           double lr_rot, double lr_trans, int wait_iters, float* best_c2w, void* stream);
+/* RO -> GO hand-off of tracking (mipsfusion.py:483-485,501-503), one 32-thread block: rot_cur (3,3) and trans_cur (3), the
+ * RandomOptimizer's state, give c2w_out (4,4) = pose_compose(rot_cur, trans_cur) and go_state (32 floats, the layout above):
+ * [0:4] matrix_to_quaternion(rot_cur) (standardised to a non-negative real part), [4:7] trans_cur, Adam moments and step
+ * count 0, [22] = -1 (no best loss yet), [23] = [24] = 0 -- what FusedPoseRefiner.refine sets up on the host. */
+int mf_track_handoff(const float* rot_cur, const float* trans_cur, float* c2w_out, float* go_state, void* stream);
 
 /* ---- keyframe pose optimisation of the mapping loop (local_BA, mipsfusion.py:259-370: get_pose_param_optim :235-241,280-282,
  * pose_optimizer.step() every pose_accum_step iterations :338-342) on the device, one thread per pose.  state (K x 24 floats):

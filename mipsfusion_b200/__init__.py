@@ -14,7 +14,7 @@ from .random_optimizer import RandomOptimizer  # noqa: F401
 from .joint_query import JointSubmapQuery, get_grid_uniform  # noqa: F401
 from .keyframe_store import KeyframeRayStore, sample_without_replacement  # noqa: F401
 from .render_full import render_full_img  # noqa: F401
-from .tracker import FusedPoseRefiner  # noqa: F401
+from .tracker import FusedPoseRefiner, FusedTracker  # noqa: F401
 from .submap_parallel import SubmapParallel  # noqa: F401
 from . import sampling_helper  # noqa: F401
 from .manager import SubmapContainment, pts_in_bbox  # noqa: F401

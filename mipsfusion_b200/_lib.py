@@ -106,6 +106,7 @@ PROTOTYPES = {
     "mf_gen_rays_packed_bwd": (_I, [_P, _P, _P, _P, _P, _L, _I, _P]),
     "mf_pose_to_c2w": (_I, [_P, _P, _P]),
     "mf_pose_refine_update": (_I, [_P, _P, _P, _P, _P, _D, _D, _I, _P, _P]),
+    "mf_track_handoff": (_I, [_P, _P, _P, _P, _P]),
     "mf_ba_pose_init": (_I, [_P, _P, _I, _P, _P, _P]),
     "mf_ba_pose_update": (_I, [_P, _P, _P, _I, _D, _D, _P, _P]),
     "mf_ro_score": (_I, [_P, _P, _P, _P, _P, _P, C.POINTER(Field), _D, _D, _I, _I, _I, _P, _P, _P, _P, _P]),

@@ -463,6 +463,34 @@ __global__ void ba_pose_update_kernel(float* __restrict__ state, float* __restri
     for (int t = 0; t < 16; ++t) dP[t] = 0.f;                            // pose_optimizer.zero_grad() after the step (:338-342)
 }
 
+// RO -> GO hand-off of tracking (mipsfusion.py:483-485,501-503): the RandomOptimizer's pose becomes c2w
+// (pose_compose, geometry_helper.py:43-47) and the GO stage's parameters (matrix_to_quaternion + translation, fresh Adam state,
+// no best loss yet), the state FusedPoseRefiner.refine builds on the host
+__global__ void track_handoff_kernel(const float* __restrict__ rot_cur, const float* __restrict__ trans_cur,
+                                     float* __restrict__ c2w, float* __restrict__ st) {
+    const int t = threadIdx.x;
+    if (t < 16) {
+        const int r = t >> 2, c = t & 3;
+        c2w[t] = r == 3 ? (c == 3 ? 1.f : 0.f) : (c == 3 ? trans_cur[r] : rot_cur[r * 3 + c]);
+    }
+    if (t != 0) return;
+    const float P[12] = {rot_cur[0], rot_cur[1], rot_cur[2], trans_cur[0], rot_cur[3], rot_cur[4], rot_cur[5], trans_cur[1],
+                         rot_cur[6], rot_cur[7], rot_cur[8], trans_cur[2]};
+    float q[4];
+    mat_to_quat(P, q);
+    for (int k = 0; k < 32; ++k) st[k] = 0.f;
+    for (int k = 0; k < 4; ++k) st[k] = q[k];
+    for (int k = 0; k < 3; ++k) st[4 + k] = P[k * 4 + 3];
+    st[22] = -1.f;
+}
+
+MF_API int mf_track_handoff(const float* rot_cur, const float* trans_cur, float* c2w_out, float* go_state, void* stream) {
+    MF_CHECK_ARG(rot_cur && trans_cur && c2w_out && go_state);
+    track_handoff_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(rot_cur, trans_cur, c2w_out, go_state);
+    MF_LAUNCH_CHECK();
+    return MF_OK;
+}
+
 MF_API int mf_ba_pose_init(const float* poses, const uint8_t* frozen, int K, float* state, float* poses_out, void* stream) {
     MF_CHECK_ARG(poses && state && poses_out && K > 0);
     ba_pose_init_kernel<<<(K + 63) / 64, 64, 0, (cudaStream_t)stream>>>(poses, frozen, K, state, poses_out);
