@@ -293,6 +293,13 @@ int mf_sample_distinct(int64_t n, int64_t k, uint32_t seed, int64_t* out, void* 
 int mf_kf_sample_rays(const float* store, int64_t n_rays, int64_t first_kf_id, const int64_t* other_kf_ids, int64_t n_other_kf,
                       int64_t last_kf_id, int n_related, int64_t n_first, int64_t n_other, int64_t n_last, uint32_t seed,
                       float* out_rays7, int64_t* out_kf_ids, int64_t* out_kf_indices, int64_t* out_idx, void* stream);
+/* The mapping batch of submap initialisation (first_frame_mapping / initialize_new_localMLP, mipsfusion.py:135-138,178,209):
+ * ray j takes pixel index i = idx[j] (idx given; each in [0, H*W)) or i = perm(j) of the mf_sample_distinct permutation of
+ * [0, H*W) with `seed` (idx NULL: the reference's random.sample(range(H*W), n)), decoded column-major h = i % H, w = i / H;
+ * out_rays7 (n,7) = [dir_cam | rgb | depth] of pixel (h, w) of the frame (dirs_cam (H*W,3), rgb (H*W,3), depth (H*W),
+ * row-major).  out_idx (optional, n) receives i.  0 <= n <= H*W; n = 0 is a no-op. */
+int mf_frame_sample_rays(const float* dirs_cam, const float* rgb, const float* depth, int img_h, int img_w, int64_t n,
+                         uint32_t seed, const int64_t* idx, float* out_rays7, int64_t* out_idx, void* stream);
 
 /* ---- gradient pose refinement of tracking (mipsfusion.py:501-556; get_pose_param_optim :235-241, qt_to_transform_matrix
  * geometry_helper.py:11-17) on the device.  state (32 floats): [0:4] quaternion (w,x,y,z), [4:7] translation, [7:14] Adam m,

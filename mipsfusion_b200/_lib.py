@@ -101,6 +101,7 @@ PROTOTYPES = {
     "mf_kf_gather_rays": (_I, [_P, _L, _L, _P, _L, _I, _P, _L, _P, _L, _P, _L, _P, _P, _P, _P]),
     "mf_sample_distinct": (_I, [_L, _L, C.c_uint32, _P, _P]),
     "mf_kf_sample_rays": (_I, [_P, _L, _L, _P, _L, _L, _I, _L, _L, _L, C.c_uint32, _P, _P, _P, _P, _P]),
+    "mf_frame_sample_rays": (_I, [_P, _P, _P, _I, _I, _L, C.c_uint32, _P, _P, _P, _P]),
     "mf_gen_rays_packed": (_I, [_P, _P, _P, _P, _P, _P, _P, _L, _I, _P]),
     "mf_gen_rays_bwd": (_I, [_P, _P, _P, _P, _P, _L, _I, _P]),
     "mf_gen_rays_packed_bwd": (_I, [_P, _P, _P, _P, _P, _L, _I, _P]),

@@ -590,3 +590,33 @@ MF_API int mf_kf_sample_rays(const float* store, int64_t n_rays, int64_t first_k
     MF_LAUNCH_CHECK();
     return MF_OK;
 }
+
+// The mapping batch of submap initialisation (first_frame_mapping / initialize_new_localMLP, mipsfusion.py:135-138,178,209):
+// random.sample(range(H*W), n) drawn as perm(j) inside the gather, decoded column-major (h = i % H, w = i / H) as the
+// reference indexes its (H, W) frame, and [dir | rgb | depth] of pixel (h, w) written to ray j.  idx: explicit draws instead.
+__global__ void frame_sample_kernel(const float* __restrict__ dirs, const float* __restrict__ rgb, const float* __restrict__ depth,
+                                    int img_h, int img_w, int64_t n, uint32_t seed, int half_bits, const int64_t* __restrict__ idx,
+                                    float* __restrict__ out, int64_t* __restrict__ out_idx) {
+    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const int64_t i = idx ? idx[j] : (int64_t)mf_feistel_perm((uint64_t)j, (uint64_t)img_h * img_w, half_bits, seed);
+    const int64_t h = i % img_h, w = i / img_h;
+    const int64_t px = h * img_w + w;
+    float* o = out + j * 7;
+    o[0] = dirs[px * 3]; o[1] = dirs[px * 3 + 1]; o[2] = dirs[px * 3 + 2];
+    o[3] = rgb[px * 3]; o[4] = rgb[px * 3 + 1]; o[5] = rgb[px * 3 + 2];
+    o[6] = depth[px];
+    if (out_idx) out_idx[j] = i;
+}
+
+MF_API int mf_frame_sample_rays(const float* dirs_cam, const float* rgb, const float* depth, int img_h, int img_w, int64_t n,
+                                uint32_t seed, const int64_t* idx, float* out_rays7, int64_t* out_idx, void* stream) {
+    MF_CHECK_ARG(img_h > 0 && img_w > 0 && n >= 0 && n <= (int64_t)img_h * img_w);
+    if (n == 0) return MF_OK;
+    MF_CHECK_ARG(dirs_cam && rgb && depth && out_rays7);
+    const int half_bits = mf_feistel_half_bits((uint64_t)img_h * img_w);
+    frame_sample_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(dirs_cam, rgb, depth, img_h, img_w, n, seed,
+                                                                                     half_bits, idx, out_rays7, out_idx);
+    MF_LAUNCH_CHECK();
+    return MF_OK;
+}

@@ -38,6 +38,42 @@ def sample_without_replacement(n, k, device, keys=None, seed=None):
     return sh._topk(ones, k, (0, 0), keys)[0]
 
 
+def frame_tensors(batch, device):
+    """batch 'direction' (1,H,W,3) | (H,W,3), 'rgb' same, 'depth' (1,H,W) | (H,W) -> (dirs (H*W,3), rgb (H*W,3), depth (H*W),
+    H, W): fp32 contiguous on ``device`` (no copy when already so)."""
+    H, W = (int(s) for s in batch["depth"].shape[-2:])
+    d = L.f32c(batch["direction"].reshape(-1, 3), device); c = L.f32c(batch["rgb"].reshape(-1, 3), device)
+    z = L.f32c(batch["depth"].reshape(-1), device)
+    if d.shape[0] != H * W or c.shape[0] != H * W or z.shape[0] != H * W:
+        raise L.MipsFusionB200Error("frame: direction, rgb and depth are not all %d x %d" % (H, W))
+    return d, c, z, H, W
+
+
+def sample_frame_rays(batch, n, device, seed=None, idx=None, out=None, out_idx=None):
+    """The mapping batch of submap initialisation (mipsfusion.py:176-180,207-211): ``n`` rays (n,7) [dir | rgb | depth] of
+    distinct pixels of a full-resolution frame (``batch`` as :meth:`KeyframeRayStore.add_keyframe` takes it), the pixel
+    index i decoded column-major (h = i % H, w = i // H) as the reference does.  The draw ``random.sample(range(H*W), n)``
+    is made inside the gather (``mf_frame_sample_rays``; ``seed`` fixes it, torch's CPU generator when None); ``idx`` gives
+    the draws instead: a host sequence is checked against [0, H*W) before it is copied, a device tensor is taken as it is.
+    ``out`` (>= n, 7) / ``out_idx`` (n,) int64: optional device buffers for the rays / the drawn indices."""
+    dev = torch.device(device)
+    d, c, z, H, W = frame_tensors(batch, dev)
+    n = int(n)
+    if idx is not None:
+        if not (isinstance(idx, torch.Tensor) and idx.is_cuda):
+            idx = torch.as_tensor(idx, dtype=torch.int64).reshape(-1)
+            if idx.numel() and (int(idx.min()) < 0 or int(idx.max()) >= H * W):
+                raise L.MipsFusionB200Error("sample_frame_rays: pixel indices outside [0, %d)" % (H * W))
+        idx = idx.to(dev, torch.int64).contiguous()
+        if idx.shape[0] != n:
+            raise L.MipsFusionB200Error("sample_frame_rays: %d indices for %d rays" % (idx.shape[0], n))
+    rays = torch.empty(n, 7, device=dev, dtype=torch.float32) if out is None else out[:n]
+    with torch.cuda.device(dev):
+        L.call("mf_frame_sample_rays", L.ptr(d), L.ptr(c), L.ptr(z), H, W, n, (_new_seed() if seed is None else int(seed)) & 0xffffffff,
+               L.ptr(idx), L.ptr(rays), L.ptr(out_idx), L.stream())
+    return rays
+
+
 class KeyframeRayStore:
     def __init__(self, config, H, W, num_kf, device):
         self.config, self.H, self.W = config, int(H), int(W)

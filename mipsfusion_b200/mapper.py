@@ -14,7 +14,7 @@ import torch
 from . import _lib as L
 from . import dist as D
 from .decoder import _Workspace
-from .keyframe_store import _new_seed
+from .keyframe_store import _new_seed, frame_tensors
 
 
 class FusedMapper:
@@ -242,11 +242,12 @@ class FusedMapper:
             D.allreduce_sum_(d_poses, self.group)
             d_poses.mul_(1.0 / self.world)
 
-    def _store_batch(self, store, first_kf_Id, related_kf_ids, pix_num, cur_rays7, **draws):
+    def _store_batch(self, store, first_kf_Id, related_kf_ids, pix_num, cur_rays7, cur=None, **draws):
         """Packed batch buffers of (pix_num, n_cur) filled from the keyframe ray store: ``pix_num`` rays of the submap's
         keyframes (:meth:`KeyframeRayStore.sample_rays_in_submap`, pose index = slot in ``related_kf_ids``), then the current
-        frame's rays ``cur_rays7`` (pose index -1 = last pose)."""
-        n_cur = 0 if cur_rays7 is None else int(cur_rays7.shape[0])
+        frame's rays (pose index -1 = last pose): ``cur_rays7``, or with ``cur`` = (frame tensors, n_cur, keys) ``n_cur`` pixels
+        of the full-resolution frame drawn as ``sample_pixels_mix(H, W, 16, 24, depth, n_cur)`` (:meth:`_draw_cur`)."""
+        n_cur = int(cur[1]) if cur is not None else 0 if cur_rays7 is None else int(cur_rays7.shape[0])
         pix_num = int(pix_num)
         R = pix_num + n_cur
         sb = self._bufs.get(("store", pix_num, n_cur))             # (keyed by the split: the tail of `idx` must stay -1)
@@ -263,10 +264,34 @@ class FusedMapper:
         else:                                                       # device draws: the gather writes straight into the batch
             store.sample_rays_in_submap(first_kf_Id, related_kf_ids, pix_num, out=sb["rays7"],
                                         out_ids=(sb["kf_ids"], sb["idx"][:pix_num]), **draws)
-        if n_cur:
+        if cur is not None:
+            self._draw_cur(cur, sb["rays7"][pix_num:])
+        elif n_cur:
             sb["rays7"][pix_num:].copy_(cur_rays7)
         self.launches += 1
         return sb
+
+    def _draw_cur(self, cur, out):
+        """The current frame's pixels of one BA iteration (mipsfusion.py:306-309): the 16 x 24 lattice, then the top
+        ``n_cur - 384`` of abs(randn) keys over the valid off-lattice pixels (``keys`` (H*W,), drawn here when None), gathered
+        into ``out`` (n_cur, 7).  Three steps on buffers that persist per (H, W, n_cur): keys, mf_sample_pixels_topk,
+        mf_kf_store."""
+        (d, c, z, H, W), n_cur, keys = cur
+        key = ("cur", H, W, n_cur)
+        cb = self._bufs.get(key)
+        if cb is None:
+            cb = self._bufs[key] = dict(keys=torch.empty(H * W, device=self.dev, dtype=torch.float32),
+                                        rows=torch.empty(n_cur, device=self.dev, dtype=torch.int64),
+                                        cols=torch.empty(n_cur, device=self.dev, dtype=torch.int64),
+                                        ws=torch.empty(int(L.lib().mf_topk_workspace_size(H * W)), device=self.dev, dtype=torch.uint8))
+        if keys is None:
+            keys = cb["keys"].normal_().abs_()                       # torch.randn_like(depth).abs() (sampling_helper.py:60)
+            self.launches += 2
+        st = L.stream()
+        L.call("mf_sample_pixels_topk", L.ptr(z), L.ptr(keys), H, W, 16, 24, n_cur, None, L.ptr(cb["rows"]), L.ptr(cb["cols"]),
+               L.ptr(cb["ws"]), st)
+        L.call("mf_kf_store", L.ptr(d), L.ptr(c), L.ptr(z), L.ptr(cb["rows"]), L.ptr(cb["cols"]), W, n_cur, L.ptr(out), st)
+        self.launches += 11                                          # lattice, top-k init, 6 radix passes, compaction, sort; gather
 
     def step_from_store(self, store, first_kf_Id, related_kf_ids, poses_all, pix_num, cur_rays7=None, EMD_w=0.01, pose_grad=False,
                         **draws):
@@ -278,8 +303,68 @@ class FusedMapper:
         sb = self._store_batch(store, first_kf_Id, related_kf_ids, pix_num, cur_rays7, **draws)
         return self._step_packed(sb, sb["idx"], poses_all, EMD_w, pose_grad)
 
+    def first_frame_mapping(self, batch, n_iters, c2w=None, pix_num=None, seed=None, u=None, EMD_w=0.01):
+        """Submap initialisation (the reference's first_frame_mapping, mipsfusion.py:155-194, and initialize_new_localMLP,
+        :198-222) on the device: ``n_iters`` map steps on one full-resolution frame, each on ``pix_num`` rays drawn afresh
+        (``mf_frame_sample_rays``: random.sample(range(H*W), pix_num) decoded column-major, gathered into the packed batch)
+        and generated with the frame's pose ``c2w`` (4,4) in the submap's frame (identity when None: the frame that opens a
+        submap defines its frame).  Map Adam runs every iteration, zero_grad fused in.
+
+        batch: as :meth:`KeyframeRayStore.add_keyframe` takes it.  pix_num: ``config["mapping"]["sample"]`` unless given.
+        seed: base of the draws (rank r, iteration i draws with seed + i world + r); from torch's CPU generator when None.
+        u: optional (n_iters, pix_num, S) stratified jitter.  A new submap is a fresh model (or ``model.recover_initial_param()``)
+        and a new FusedMapper, whose Adam state starts at zero as the reference's create_optimizer's does.  With a process
+        group the step's data-parallel exchange applies and every rank draws its own rays.
+
+        -> losses (n_iters, 8) device tensor, overwritten by the next call of the same shape; the model is stepped in place.
+        No host synchronisation; no allocation after the first call for an (H, W, pix_num, n_iters) when the inputs are
+        float32, contiguous and on the device."""
+        n_iters = int(n_iters)
+        if n_iters < 0:
+            raise L.MipsFusionB200Error("first_frame_mapping: n_iters must be >= 0, got %d" % n_iters)
+        if pix_num is None:
+            mc = self.model.config.get("mapping", {})
+            if "sample" not in mc:
+                raise L.MipsFusionB200Error("first_frame_mapping: pix_num not given and config['mapping'] has no 'sample'")
+            pix_num = mc["sample"]
+        R = int(pix_num)
+        d, c, z, H, W = frame_tensors(batch, self.dev)
+        if not 0 < R <= H * W:
+            raise L.MipsFusionB200Error("first_frame_mapping: pix_num must lie in [1, H*W = %d], got %d" % (H * W, R))
+        losses = self._bufs.get(("init_losses", R, n_iters))
+        if losses is None:
+            losses = self._bufs[("init_losses", R, n_iters)] = torch.zeros(n_iters, 8, device=self.dev, dtype=torch.float32)
+        if n_iters == 0:
+            return losses
+        sb = self._bufs.get(("frame", R))
+        if sb is None:
+            f32 = dict(device=self.dev, dtype=torch.float32)
+            sb = self._bufs[("frame", R)] = dict(rays7=torch.empty(R, 7, **f32), o=torch.empty(R, 3, **f32), d=torch.empty(R, 3, **f32),
+                                                 rgb=torch.empty(R, 3, **f32), depth=torch.empty(R, **f32))
+        if c2w is None:
+            P = self._bufs.get("eye")
+            if P is None:
+                P = self._bufs["eye"] = torch.eye(4, device=self.dev, dtype=torch.float32)[None]
+        else:
+            P = torch.as_tensor(c2w).reshape(1, 4, 4)
+            if not (P.is_cuda and P.dtype == torch.float32 and P.is_contiguous()):
+                P = P.to(self.dev, torch.float32).contiguous()      # once, not per iteration
+        if u is not None:
+            u = L.f32c(u, self.dev)
+        self.model.decoder.prepared()                                # adopt external writes to the decoder's parameters
+        seed = _new_seed() if seed is None else int(seed)
+        world, rank = D.world(self.group)
+        st = L.stream()
+        for i in range(n_iters):
+            L.call("mf_frame_sample_rays", L.ptr(d), L.ptr(c), L.ptr(z), H, W, R, (seed + i * world + rank) & 0xffffffff, None,
+                   L.ptr(sb["rays7"]), None, st)
+            li = self._step_packed(sb, None, P, EMD_w, False, u=None if u is None else u[i])
+            losses[i].copy_(li)
+            self.launches += 2
+        return losses
+
     def local_ba(self, store, first_kf_Id, related_kf_ids, poses_all, pix_num, cur_rays7=None, n_iters=None, pose_accum_step=None,
-                 lr_rot=None, lr_trans=None, optim_cur=None, seed=None, u=None, EMD_w=0.01):
+                 lr_rot=None, lr_trans=None, optim_cur=None, seed=None, u=None, EMD_w=0.01, cur_frame=None, n_cur=None, cur_keys=None):
         """The reference's local bundle adjustment (MIPSFusion.local_BA, mipsfusion.py:259-370; the same body runs in
         InactiveMap.local_BA, local_BA_switch and initialize_new_localMLP) on the device: ``n_iters`` mapping iterations fed from
         the keyframe ray store (as :meth:`step_from_store`) that also accumulate d loss / d poses, and every ``pose_accum_step``
@@ -294,8 +379,13 @@ class FusedMapper:
         stratified jitter.  With a process group every rank draws its own rays and the pose gradients are averaged over the
         ranks once per pose step, so all ranks hold the same poses.
 
+        The current frame's rays: ``cur_rays7`` (n,7), the same rows in every iteration; or ``cur_frame`` (a batch dict as
+        :meth:`KeyframeRayStore.add_keyframe` takes it) with ``n_cur``: every iteration draws ``n_cur`` pixels of it afresh as
+        the reference's ``sample_pixels_mix(H, W, 16, 24, depth, n_cur)`` does (mipsfusion.py:306-309), on abs(randn) keys
+        drawn on the device or from ``cur_keys[i]`` (cur_keys (n_iters, H*W)).  384 <= n_cur <= 384 + 4096.
+
         -> (poses (K,4,4), losses (n_iters, 8)) device tensors, overwritten by the next call of the same shape.  No host
-        synchronisation; no allocation after the first call for a (K, pix_num, n_cur, n_iters)."""
+        synchronisation; no allocation after the first call for a (K, pix_num, n_cur, n_iters) (and frame size)."""
         mc = self.model.config.get("mapping", {})
 
         def hp(v, key):
@@ -308,9 +398,27 @@ class FusedMapper:
         lr_rot, lr_trans, optim_cur = float(hp(lr_rot, "lr_rot")), float(hp(lr_trans, "lr_trans")), bool(hp(optim_cur, "optim_cur"))
         if accum < 1:
             raise L.MipsFusionB200Error("local_ba: pose_accum_step must be >= 1")
+        cur = None
+        if cur_frame is None and (n_cur is not None or cur_keys is not None):
+            raise L.MipsFusionB200Error("local_ba: n_cur / cur_keys are for the cur_frame draw; cur_frame is missing")
+        if cur_frame is not None:
+            if cur_rays7 is not None:
+                raise L.MipsFusionB200Error("local_ba: pass cur_rays7 or cur_frame, not both")
+            if n_cur is None:
+                raise L.MipsFusionB200Error("local_ba: cur_frame needs n_cur")
+            n_cur = int(n_cur)
+            if n_cur < 16 * 24 or n_cur - 16 * 24 > 4096:
+                raise L.MipsFusionB200Error("local_ba: n_cur must lie in [384, 4480] (the 16 x 24 lattice plus at most 4096 "
+                                            "random pixels), got %d" % n_cur)
+            frame = frame_tensors(cur_frame, self.dev)
+            if cur_keys is not None:
+                cur_keys = L.f32c(cur_keys, self.dev)
+                if tuple(cur_keys.shape) != (n_iters, frame[3] * frame[4]):
+                    raise L.MipsFusionB200Error("local_ba: cur_keys must be (n_iters, H*W) = (%d, %d)" % (n_iters, frame[3] * frame[4]))
+            cur = (frame, n_cur, cur_keys)
         self.model.decoder.prepared()                                # adopt external writes to the decoder's parameters
         K = int(poses_all.shape[0])
-        n_cur = 0 if cur_rays7 is None else int(cur_rays7.shape[0])
+        n_cur = int(n_cur) if cur is not None else 0 if cur_rays7 is None else int(cur_rays7.shape[0])
         key = ("ba", K, int(pix_num), n_cur)
         bb = self._bufs.get(key)
         if bb is None:
@@ -336,7 +444,9 @@ class FusedMapper:
         seed = _new_seed() if seed is None else int(seed)
         world, rank = D.world(self.group)
         for i in range(n_iters):
-            sb = self._store_batch(store, first_kf_Id, related_kf_ids, pix_num, cur_rays7, seed=(seed + 3 * (i * world + rank)) & 0xffffffff)
+            ci = None if cur is None else (cur[0], cur[1], None if cur[2] is None else cur[2][i])
+            sb = self._store_batch(store, first_kf_Id, related_kf_ids, pix_num, cur_rays7, cur=ci,
+                                   seed=(seed + 3 * (i * world + rank)) & 0xffffffff)
             li, _ = self._step_packed(sb, sb["idx"], bb["poses"], EMD_w, True, u=None if u is None else L.f32c(u[i], self.dev),
                                       d_poses=bb["d_poses"])
             losses[i].copy_(li)
