@@ -146,7 +146,8 @@ int mf_mlp_bwd(const float* embed, const float* embed_pos, const float* pts, con
  * pts (N,3) fp32 in the submap frame -> out (N,10).  normalize=0 skips the bound normalisation
  * (query_color_sdf called directly on pre-normalised points, as model/Mesher.py:487 does). */
 int mf_field_query(const float* pts, const mf_field* field_host, int normalize, float* out, int64_t N, void* stream);
-/* backward of the above: grad_grid/grad_mlp accumulate; d_pts (N,3) optional.
+/* backward of the above: grad_grid/grad_mlp accumulate; d_pts (N,3) optional.  grad_grid = grad_mlp = NULL: point gradients
+ * only (d_pts required; no weight gradients, no grid scatter; fp32 or tensor-core decoder as the field selects).
  * workspace: mf_field_bwd_workspace_size(N, 0) floats (per-CTA partial sums + the list of points whose d_out row is
  * non-zero: rows that are exactly zero add nothing to any gradient and are skipped). */
 int64_t mf_field_bwd_workspace_size(int64_t n_points, int want_ray_grads);
@@ -425,6 +426,31 @@ int mf_mcubes_mesh(const void* count_workspace, int64_t nx, int64_t ny, int64_t 
 int mf_mesh_seen_mask(const float* points, int64_t n, const float* w2c, const float* max_depth, int k, const float* K, int img_w,
                       int img_h, int edge, uint8_t* seen, void* stream);
 int mf_mesh_face_mask(const uint8_t* seen, const int64_t* faces, int64_t n_faces, uint8_t* keep, void* stream);
+
+/* ---- a15: overlap-region SDF consistency of the inactive-map global BA (InactiveMap.py:128-139 infer_pts, :149-165
+ * get_SDF_dif, :177-192 get_SDF_dif2; loss helper_functions/geometry_helper.py:225-229), P submap pairs x N rays ----
+ * pair_tab (P,4) int32 device: {pose1, pose2, off1, off2} = rows of the two first-keyframe poses in first_poses (K,4,4) and
+ * the first row of each side's N points in pts / raw / d_raw / d_pts (2 P N rows in all, grouped by submap by the caller).
+ * Element (p, r) of target_d is target_d[(p N + r) ld_d], its direction rays_d_cam[(p N + r) ld_dir + 0..2].  ovlp: the
+ * overlap keyframe poses, (P, N, 4, 4) when ovlp_per_ray, else (P, 1, 4, 4).  All fp32 device, no atomics (deterministic).
+ * mf_overlap_points: finv (P,2,16) = first_poses[pose_s]^-1 (fp64 adjugate / determinant, rounded once to fp32);
+ *   A = finv O (fp32), pts[off_s + r] = A[:3,3] + (sum_k d_cam[k] A[:3,k]) depth (InactiveMap.py:128-139). */
+int mf_overlap_points(const float* first_poses, const int* pair_tab, int P, int N, const float* ovlp, int ovlp_per_ray,
+                      const float* target_d, int ld_d, const float* rays_d_cam, int ld_dir, float* finv, float* pts, void* stream);
+/* mf_overlap_loss: raw = the field outputs of pts (mf_field_query, per submap segment); sdf = raw[:,3] trunc;
+ * loss[p] = sum_r (sdf1 m - sdf2 m)^2 / (count_nonzero(m) + 0.001) (geometry_helper.py:225-229), fixed-order reduction.
+ * mask_kind 0: m = (target_d > 0) (get_SDF_dif, InactiveMap.py:149-165); 1: float mask[(p N + r) ld_m]; 2: uint8/bool mask
+ * (get_SDF_dif2, :177-192).  d_raw (2 P N, 10): d loss[p] / d raw for an upstream gradient of 1, only column 3 non-zero,
+ * rows with m = 0 exactly zero (the field backward skips them). */
+int mf_overlap_loss(const float* raw, const int* pair_tab, int P, int N, const float* target_d, int ld_d, const void* mask,
+                    int mask_kind, int ld_m, double trunc, float* loss, float* d_raw, void* stream);
+/* mf_overlap_pose_bwd: d_pts = mf_field_query_bwd of d_raw (point gradients only); g_loss[p ld_g] the upstream gradient of
+ * loss[p] (ld_g = 0: one shared value; NULL = 1).  dA = d loss / d A (dA[:3,3] = dx, dA[i][k] = dx_i depth d_cam_k); dF_pair (P,2,16) scratch receives
+ * -finv^T (sum_r dA_r O_r^T) finv^T; d_first (n_poses,4,4) = sum over pairs in pair order (side 1, then side 2) of the sides
+ * that use each pose (written, not accumulated); d_ovlp (same shape as ovlp, optional) = sum_s finv_s^T dA_s. */
+int mf_overlap_pose_bwd(const float* finv, const int* pair_tab, int P, int N, const float* ovlp, int ovlp_per_ray,
+                        const float* target_d, int ld_d, const float* rays_d_cam, int ld_dir, const float* d_pts,
+                        const float* g_loss, int ld_g, int n_poses, float* dF_pair, float* d_first, float* d_ovlp, void* stream);
 
 #ifdef __cplusplus
 }

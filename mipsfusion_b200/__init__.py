@@ -16,6 +16,7 @@ from .keyframe_store import KeyframeRayStore, sample_without_replacement  # noqa
 from .render_full import render_full_img  # noqa: F401
 from .tracker import FusedPoseRefiner, FusedTracker  # noqa: F401
 from .submap_parallel import SubmapParallel  # noqa: F401
+from .overlap import OverlapSDF  # noqa: F401
 from . import sampling_helper  # noqa: F401
 from .manager import SubmapContainment, pts_in_bbox  # noqa: F401
 from . import marching_cubes  # noqa: F401  (module, like the reference's `marching_cubes` package: marching_cubes.marching_cubes(volume, isovalue, truncation))

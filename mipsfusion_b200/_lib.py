@@ -124,6 +124,9 @@ PROTOTYPES = {
     "mf_mcubes_mesh": (_I, [_P, _L, _L, _L, C.c_float, _L, _P, _P, _P, _P, _P]),
     "mf_mesh_seen_mask": (_I, [_P, _L, _P, _P, _I, _P, _I, _I, _I, _P, _P]),
     "mf_mesh_face_mask": (_I, [_P, _P, _L, _P, _P]),
+    "mf_overlap_points": (_I, [_P, _P, _I, _I, _P, _I, _P, _I, _P, _I, _P, _P, _P]),
+    "mf_overlap_loss": (_I, [_P, _P, _I, _I, _P, _I, _P, _I, _I, _D, _P, _P, _P]),
+    "mf_overlap_pose_bwd": (_I, [_P, _P, _I, _I, _P, _I, _P, _I, _P, _I, _P, _P, _I, _I, _P, _P, _P, _P]),
 }
 
 _lib = None

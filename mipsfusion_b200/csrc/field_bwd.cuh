@@ -34,7 +34,8 @@ __device__ __forceinline__ void head_backward_tile(const float* __restrict__ d_r
 // Full decoder backward for one tile.  On entry: E, G, H1, H2, H3, OUT hold the forward
 // activations and DZ the head gradients.  On exit: G rows hold dL/dgrid-features, and (WANT_DX)
 // E rows hold dL/de.  gpart is this CTA's private partial of the parameter gradient blob.
-template <bool WANT_DX>
+// PARAMS = false (with WANT_DX): input gradients only, no weight or bias gradients (gpart unused).
+template <bool WANT_DX, bool PARAMS = true>
 __device__ __forceinline__ void mlp_backward_tile(const float* __restrict__ prep, float* sm, float* __restrict__ gpart) {
     const int tid = threadIdx.x, tx = tid & 15, m0 = (tid >> 4) * 4;
     float* E = sm + ROW_E * LDA; float* G = sm + ROW_G * LDA;
@@ -42,7 +43,7 @@ __device__ __forceinline__ void mlp_backward_tile(const float* __restrict__ prep
     float* DZ = sm + ROW_DZ * LDA;
 
     // ---- weight gradients of the two small heads -------------------------------------------------
-    {   // sdf_linear.2: dW[c][k] += sum_m DZ[c][m] H3[k][m]   (5 x 128): thread (k = tid & 127, half)
+    if (PARAMS) {   // sdf_linear.2: dW[c][k] += sum_m DZ[c][m] H3[k][m]   (5 x 128): thread (k = tid & 127, half)
         const int k = tid & 127, half = tid >> 7;
         const int c0 = half ? 3 : 0, c1 = half ? 5 : 3;
         float s[3] = {0.f, 0.f, 0.f};
@@ -98,9 +99,11 @@ __device__ __forceinline__ void mlp_backward_tile(const float* __restrict__ prep
     __syncthreads();
 
     // ---- sdf_linear.0: wgrad (128 x 96) on A3 = [H2[0..63], G], bias ------------------------------
-    wgrad_tile<6>(H3, [&](int k) -> const float* { return k < 64 ? H2 + k * LDA : G + (k - 64) * LDA; }, D_SDF_IN,
-                  gpart + OFF_WS1, tid);
-    bias_grad_tile(H3, gpart + OFF_BS1, tid);
+    if (PARAMS) {
+        wgrad_tile<6>(H3, [&](int k) -> const float* { return k < 64 ? H2 + k * LDA : G + (k - 64) * LDA; }, D_SDF_IN,
+                      gpart + OFF_WS1, tid);
+        bias_grad_tile(H3, gpart + OFF_BS1, tid);
+    }
     {   // dgrad: dA3[k][m] = sum_n Ws1[n][k] dZ3[n][m], k < 96 (registers; written after the barrier)
         float acc[4][6];
 #pragma unroll
@@ -119,8 +122,10 @@ __device__ __forceinline__ void mlp_backward_tile(const float* __restrict__ prep
     __syncthreads();
 
     // ---- pts_linear.2: wgrad (128 x 128) with dH = H2, A = H1; dgrad -> dZ1 in place of H1 -------
-    wgrad_tile<8>(H2, [&](int k) -> const float* { return H1 + k * LDA; }, D_H, gpart + OFF_W2, tid);
-    bias_grad_tile(H2, gpart + OFF_B2, tid);
+    if (PARAMS) {
+        wgrad_tile<8>(H2, [&](int k) -> const float* { return H1 + k * LDA; }, D_H, gpart + OFF_W2, tid);
+        bias_grad_tile(H2, gpart + OFF_B2, tid);
+    }
     {
         float acc[4][8];
 #pragma unroll
@@ -140,8 +145,10 @@ __device__ __forceinline__ void mlp_backward_tile(const float* __restrict__ prep
     __syncthreads();
 
     // ---- pts_linear.0: wgrad (128 x 51) with dZ1 = H1, A = E; optional dgrad -> dE ----------------
-    wgrad_tile<4>(H1, [&](int k) -> const float* { return E + k * LDA; }, D_E, gpart + OFF_W1, tid);
-    bias_grad_tile(H1, gpart + OFF_B1, tid);
+    if (PARAMS) {
+        wgrad_tile<4>(H1, [&](int k) -> const float* { return E + k * LDA; }, D_E, gpart + OFF_W1, tid);
+        bias_grad_tile(H1, gpart + OFF_B1, tid);
+    }
     if (WANT_DX) {
         float acc[4][4];
 #pragma unroll
@@ -172,7 +179,8 @@ __device__ __forceinline__ void mlp_backward_tile(const float* __restrict__ prep
 // Encoder backward: scatter dL/dgrid-features (G rows) into grad_grid and, if WANT_DX, gather
 // dL/dx from the grid levels, the frequency features and the raw xyz input; the four partial
 // sums per point are combined through the PS rows and converted to dL/dp by the source.
-template <class Src, bool WANT_DX>
+// PARAMS = false: no scatter into grad_grid (input gradients only).
+template <class Src, bool WANT_DX, bool PARAMS = true>
 __device__ __forceinline__ void encode_backward_tile(const FieldDev& f, const Src& src, int64_t tile, int64_t N,
                                                      float* sm, float* __restrict__ grad_grid,
                                                      float* __restrict__ d_pts,
@@ -191,7 +199,7 @@ __device__ __forceinline__ void encode_backward_tile(const FieldDev& f, const Sr
         for (int ll = 0; ll < 4; ++ll) {
             const int l = q * 4 + ll;
             const float2 dy = make_float2(G[(2 * l) * LDA + m], G[(2 * l + 1) * LDA + m]);
-            grid_level_bwd<WANT_DX>(x, dy, grid2, grad_grid, level_info(f, l), dx);
+            grid_level_bwd<WANT_DX, PARAMS>(x, dy, grid2, grad_grid, level_info(f, l), dx);
         }
     }
     if (WANT_DX) {

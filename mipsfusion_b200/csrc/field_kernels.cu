@@ -127,6 +127,28 @@ __global__ void __launch_bounds__(NT, 1) field_bwd_kernel(FieldDev f, Src src, c
     }
 }
 
+// Input gradients only on the fp32 decoder (no weight gradients, no grid scatter): the pose gradients of the overlap-region
+// SDF consistency (overlap_kernels.cu), whose residual is a small difference of two fields and needs the fp32 recomputation.
+// Every point's d_pts depends on that point and its d_raw row alone (no atomics): deterministic.
+template <class Src>
+__global__ void __launch_bounds__(NT, 1) field_bwd_dx_kernel(FieldDev f, Src src, const float* __restrict__ d_raw,
+                                                             float* __restrict__ d_pts, int64_t N_all, ActiveMap am) {
+    extern __shared__ __align__(16) float sm[];
+    const int64_t N = am.n(N_all);
+    const int64_t n_tiles = (N + TP - 1) / TP;
+    for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+        encode_tile(f, src, tile, N, sm, am);
+        __syncthreads();
+        mlp_forward_tile<false>(f.prep, sm, sm + ROW_H3 * LDA);
+        __syncthreads();
+        head_backward_tile(d_raw, tile, N, sm, am);
+        __syncthreads();
+        mlp_backward_tile<true, false>(f.prep, sm, nullptr);
+        encode_backward_tile<Src, true, false>(f, src, tile, N, sm, nullptr, d_pts, am);
+        __syncthreads();
+    }
+}
+
 template <bool WANT_DX>
 __global__ void __launch_bounds__(NT, 1) mlp_bwd_kernel(const float* embed, const float* embed_pos, const float* pts,
                                                         const float* __restrict__ prep, const float* __restrict__ d_out,
@@ -558,10 +580,17 @@ static int launch_field_bwd(const FieldDev& d, const Src& src, const float* d_ra
     ActiveMap am{nullptr, nullptr};
     int rc0 = compact_active_points(d_raw, N, scratch, &am, st); if (rc0) return rc0;
     if (d_pts) MF_CUDA(cudaMemsetAsync(d_pts, 0, (size_t)N * 3 * sizeof(float), st));   // skipped points: exactly zero
-    const bool params = grad_grid != nullptr;          // false: input gradients only (pose refinement)
-    if (!params && (d.impl == 1 || !d_pts)) {
-        mf_set_error("backward without parameter gradients needs the tensor-core decoder and a ray / point gradient output");
+    const bool params = grad_grid != nullptr;          // false: input gradients only (pose refinement, overlap consistency)
+    if (!params && !d_pts) {
+        mf_set_error("backward without parameter gradients needs a ray / point gradient output");
         return MF_ERR_INVALID;
+    }
+    if (!params && d.impl == 1) {
+        const int grid = persistent_grid(N, 1);
+        int rc = set_smem(field_bwd_dx_kernel<Src>, SMEM_BWD); if (rc) return rc;
+        field_bwd_dx_kernel<Src><<<grid, NT, SMEM_BWD, st>>>(d, src, d_raw, d_pts, N, am);
+        MF_LAUNCH_CHECK();
+        return MF_OK;
     }
     if (d.impl != 1) {                                 // tcgen05 path: 128-point tiles, one CTA per SM
         const int64_t tiles = (N + TC_TP - 1) / TC_TP;
@@ -631,7 +660,9 @@ MF_API int mf_field_query_bwd(const float* pts, const mf_field* field, int norma
                               float* grad_mlp, float* d_pts, float* workspace, int64_t N, void* stream) {
     MF_CHECK_ARG(N >= 0);
     if (N == 0) return MF_OK;
-    MF_CHECK_ARG(pts && d_out && grad_grid && grad_mlp && workspace);
+    MF_CHECK_ARG(pts && d_out && workspace);
+    MF_CHECK_ARG((grad_grid == nullptr) == (grad_mlp == nullptr));      // both NULL: point gradients only (needs d_pts)
+    MF_CHECK_ARG(grad_grid || d_pts);
     MF_CHECK_ARG(((uintptr_t)grad_grid & 15) == 0);          // the scatter uses 16-byte reductions
     FieldDev d; int rc = mf_field_to_dev(field, &d); if (rc) return rc;
     SrcPoints src{pts, normalize};
