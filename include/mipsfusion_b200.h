@@ -90,6 +90,10 @@ int mf_set_dynamic_tiles(int on);
 /* Number of SMs the forward kernel leaves free (default 0).  The data-parallel mapper sets 1 so that its count all-reduce, issued
  * on the collective library's stream, overlaps the forward instead of waiting for an SM. */
 int mf_set_sm_reserve(int n);
+/* Programmatic dependent launch of the map step's kernels: 1 = on (default unless MF_NO_PDL=1 in the environment), 0 = plain
+ * stream order.  Process-wide; results are identical either way (A/B switch). */
+int mf_set_pdl(int on);
+int mf_get_pdl(void);
 int mf_tc_check_error(void);
 /* Diagnostics: out (128,128) = x (128,K) w (128,K)^T through one tcgen05 layer; K % 16 == 0, K <= 128;
  * passes = 1 (bf16) or 3 (bf16x3 split). */

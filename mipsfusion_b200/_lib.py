@@ -58,6 +58,8 @@ PROTOTYPES = {
     "mf_set_bwd_impl": (_I, [_I]),
     "mf_set_dynamic_tiles": (_I, [_I]),
     "mf_set_sm_reserve": (_I, [_I]),
+    "mf_set_pdl": (_I, [_I]),
+    "mf_get_pdl": (_I, []),
     "mf_containment": (_I, [_P, _P, _P, _P, _P, _P, _I, _L, _I, _P, _P, _P]),
     "mf_tc_check_error": (_I, []),
     "mf_debug_umma_linear": (_I, [_P, _P, _P, _I, _I, _P]),

@@ -82,6 +82,7 @@ __device__ __forceinline__ void mlp_prepare_tc(const float* __restrict__ mlp, ui
 constexpr int PREP_BLOCKS_SIMT = (PREP_SIMT_SIZE + 255) / 256;
 constexpr int PREP_BLOCKS_TC = (128 * 320 + F_COUNT + 255) / 256;
 __global__ void __launch_bounds__(256) mlp_prepare_kernel(const float* __restrict__ mlp, float* __restrict__ prep) {
+    mf_pdl_wait(); mf_pdl_trigger();
     if (blockIdx.x < PREP_BLOCKS_SIMT) mlp_prepare_simt(mlp, prep, blockIdx.x * 256 + threadIdx.x);
     else mlp_prepare_tc(mlp, reinterpret_cast<uint8_t*>(prep + PREP_TC), (blockIdx.x - PREP_BLOCKS_SIMT) * 256 + threadIdx.x);
 }
@@ -195,6 +196,7 @@ __global__ void __launch_bounds__(NT, 1) mlp_bwd_kernel(const float* embed, cons
 __global__ void __launch_bounds__(256) reduce_partials_kernel(const float* __restrict__ part, int n_cta, float* __restrict__ grad_mlp,
                                                               int transposed, const float* __restrict__ mlp) {
     __shared__ float acc[8][32];
+    mf_pdl_wait(); mf_pdl_trigger();
     if (transposed == 2 && blockIdx.x == gridDim.x - 1) {
         __shared__ float dbs1[D_H], dbr[4];
         const int t = threadIdx.x;
@@ -446,8 +448,7 @@ MF_API int64_t mf_mlp_prep_size(void) { return PREP_SIZE; }
 
 MF_API int mf_mlp_prepare(const float* mlp, float* mlp_prep, void* stream) {
     MF_CHECK_ARG(mlp && mlp_prep);
-    mlp_prepare_kernel<<<PREP_BLOCKS_SIMT + PREP_BLOCKS_TC, 256, 0, (cudaStream_t)stream>>>(mlp, mlp_prep);
-    MF_LAUNCH_CHECK();
+    MF_CUDA(mf_launch(mlp_prepare_kernel, PREP_BLOCKS_SIMT + PREP_BLOCKS_TC, 256, 0, (cudaStream_t)stream, mlp, mlp_prep));
     return MF_OK;
 }
 
@@ -496,6 +497,7 @@ constexpr int ACT_BLK = 1024;
 
 __global__ void __launch_bounds__(ACT_BLK) active_count_kernel(const float* __restrict__ d_raw, int64_t N,
                                                                uint32_t* __restrict__ flags, int* __restrict__ blk_cnt) {
+    mf_pdl_wait(); mf_pdl_trigger();
     const int64_t i = (int64_t)blockIdx.x * ACT_BLK + threadIdx.x;
     bool on = false;
     if (i < N) {
@@ -513,6 +515,7 @@ __global__ void __launch_bounds__(ACT_BLK) active_fill_kernel(const uint32_t* __
                                                               int* __restrict__ idx, int* __restrict__ n_active) {
     __shared__ int wsum[32];
     __shared__ int base_s;
+    mf_pdl_wait(); mf_pdl_trigger();
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     int part = 0;
     for (int j = tid; j < (int)blockIdx.x; j += ACT_BLK) part += blk_cnt[j];
@@ -557,10 +560,8 @@ static int compact_active_points(const float* d_raw, int64_t N, float* scratch, 
     uint32_t* flags = reinterpret_cast<uint32_t*>(idx + N);
     int* blk_cnt = reinterpret_cast<int*>(flags + nb * 32);
     int* count = blk_cnt + nb;
-    active_count_kernel<<<(unsigned)nb, ACT_BLK, 0, st>>>(d_raw, N, flags, blk_cnt);
-    MF_LAUNCH_CHECK();
-    active_fill_kernel<<<(unsigned)nb, ACT_BLK, 0, st>>>(flags, blk_cnt, idx, count);
-    MF_LAUNCH_CHECK();
+    MF_CUDA(mf_launch(active_count_kernel, (unsigned)nb, ACT_BLK, 0, st, d_raw, N, flags, blk_cnt));
+    MF_CUDA(mf_launch(active_fill_kernel, (unsigned)nb, ACT_BLK, 0, st, flags, blk_cnt, idx, count));
     am->idx = idx; am->count = count;
     return MF_OK;
 }
@@ -611,13 +612,12 @@ static int launch_field_bwd(const FieldDev& d, const Src& src, const float* d_ra
                 field_bwd_tc3_kernel<Src><<<grid, b3::B3_NT, b3::SMEM, st>>>(d, src, d_raw, grad_grid, workspace, cta_scr, N, am, mf_tc_error_flag(), mf_tc_profile_buffer());
             } else {                                       // three roles (default)
                 int rc = set_smem(field_bwd_tc2_kernel<Src>, b2::SMEM); if (rc) return rc;
-                field_bwd_tc2_kernel<Src><<<grid, b2::B2_NT, b2::SMEM, st>>>(d, src, d_raw, grad_grid, workspace, cta_scr, N, am, mf_tc_error_flag(), mf_tc_profile_buffer(),
-                                                                             mf_bwd_impl() == 2 ? 0 : 1);
+                MF_CUDA(mf_launch(field_bwd_tc2_kernel<Src>, grid, b2::B2_NT, b2::SMEM, st, d, src, d_raw, grad_grid, workspace, cta_scr, N, am,
+                                  mf_tc_error_flag(), mf_tc_profile_buffer(), mf_bwd_impl() == 2 ? 0 : 1));
             }
             mf_ktimer_end(1, st);
             MF_LAUNCH_CHECK();
-            reduce_partials_kernel<<<(MF_MLP_PARAMS + 31) / 32 + 1, 256, 0, st>>>(workspace, grid, grad_mlp, 2, d.prep);
-            MF_LAUNCH_CHECK();
+            MF_CUDA(mf_launch(reduce_partials_kernel, (MF_MLP_PARAMS + 31) / 32 + 1, 256, 0, st, workspace, grid, grad_mlp, 2, d.prep));
             return MF_OK;
         }
         if (d_pts) {

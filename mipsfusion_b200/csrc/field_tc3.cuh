@@ -93,6 +93,7 @@ __global__ void __launch_bounds__(2 * T3_GT, 1) field_fwd_tc3_kernel(FieldDev f,
     __shared__ uint32_t tmem_ptr_s;
     // profiling stamps (mf_debug_profile): CTA 0, third tile; producers -> prof[40..], consumers -> prof[48..]
 #define T3_MARK(slot) do { if (prof && blockIdx.x == 0 && tid == 0 && k == 2) prof[slot] = clock64(); } while (0)
+    mf_pdl_wait();                                       // (programmatic launch, mf_common.cuh: no global access before it)
     if (n_dev) N = (int64_t)*n_dev;
     if (prof && blockIdx.x == 0 && threadIdx.x == 0) prof[29] = clock64();
     if (prof && threadIdx.x == 0 && blockIdx.x < 256) prof[64 + 2 * blockIdx.x] = mf_globaltimer();
@@ -389,6 +390,7 @@ __global__ void __launch_bounds__(2 * T3_GT, 1) field_fwd_tc3_kernel(FieldDev f,
         ok = c.ok;
     }
     if (!ok && err) atomicExch(err, 1);
+    mf_pdl_trigger();                                    // every tile of this CTA is drawn: the next kernel may start its prologue
     umma::fence_before_sync();
     __syncthreads();
     if (prof && blockIdx.x == 0 && threadIdx.x == 0) prof[28] = clock64();

@@ -185,6 +185,7 @@ __global__ void __launch_bounds__(b2::B2_NT, 1) field_bwd_tc2_kernel(FieldDev f,
     using namespace b2;
     extern __shared__ uint8_t smem_raw[];
     const int tid = threadIdx.x, warp = tid >> 5;
+    mf_pdl_wait();                                       // (programmatic launch, mf_common.cuh: no global access before it)
     if (prof && tid == 0 && blockIdx.x < 256) prof[576 + 2 * blockIdx.x] = mf_globaltimer();
     float* gpart = part + (size_t)blockIdx.x * MF_MLP_PARAMS;
     for (int i = tid; i < MF_MLP_PARAMS; i += B2_NT) gpart[i] = 0.f;
@@ -761,6 +762,7 @@ __global__ void __launch_bounds__(b2::B2_NT, 1) field_bwd_tc2_kernel(FieldDev f,
     }
 #undef B2_MARK
     if (!c.ok && err) atomicExch(err, 1);
+    mf_pdl_trigger();                                    // every tile of this CTA is done: the next kernel may start its prologue
     umma::fence_before_sync();
     __syncthreads();
     if (prof && tid == 0 && blockIdx.x < 256) prof[577 + 2 * blockIdx.x] = mf_globaltimer();

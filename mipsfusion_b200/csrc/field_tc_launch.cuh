@@ -38,9 +38,8 @@ static inline int launch_field_fwd_tc3(const FieldDev& d, const Src& src, const 
     const int64_t tiles = (N + TC_TP - 1) / TC_TP;
     const int64_t cap = mf_sm_count_cached() - mf_sm_reserve() > 0 ? mf_sm_count_cached() - mf_sm_reserve() : 1;
     const int grid = (int)(tiles < cap ? (tiles > 0 ? tiles : 1) : cap);
-    field_fwd_tc3_kernel<Src, Epi, SDF_ONLY><<<grid, 2 * T3_GT, SMEM_TC3, st>>>(d, src, epi, N, n_dev, d.tc_img, mf_tc_error_flag(), mf_tc_profile_buffer(),
-                                                                              mf_tile_counter());
-    MF_LAUNCH_CHECK();
+    MF_CUDA(mf_launch(field_fwd_tc3_kernel<Src, Epi, SDF_ONLY>, grid, 2 * T3_GT, SMEM_TC3, st, d, src, epi, N, n_dev, d.tc_img,
+                      mf_tc_error_flag(), mf_tc_profile_buffer(), mf_tile_counter()));
     return MF_OK;
 }
 

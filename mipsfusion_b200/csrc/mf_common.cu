@@ -1,5 +1,6 @@
 // Error reporting and device-attribute cache for the C ABI.
 #include <stdarg.h>
+#include <stdlib.h>
 
 #include "mf_common.cuh"
 
@@ -87,6 +88,22 @@ MF_API int mf_set_dynamic_tiles(int on) {
     g_dynamic_tiles = on ? 1 : 0;
     return MF_OK;
 }
+
+// Programmatic dependent launch of the map step's kernels (mf_launch, mf_common.cuh): on unless MF_NO_PDL=1; mf_set_pdl switches
+// it at run time (A/B of both launch modes in one process).
+static int g_pdl = -1;
+bool mf_pdl_enabled() {
+    if (g_pdl < 0) {
+        const char* e = getenv("MF_NO_PDL");
+        g_pdl = (e && e[0] && strcmp(e, "0") != 0) ? 0 : 1;
+    }
+    return g_pdl != 0;
+}
+MF_API int mf_set_pdl(int on) {
+    g_pdl = on ? 1 : 0;
+    return MF_OK;
+}
+MF_API int mf_get_pdl(void) { return mf_pdl_enabled() ? 1 : 0; }
 
 static int* g_tc_err[64] = {nullptr};
 int* mf_tc_error_flag() {

@@ -30,6 +30,41 @@ void mf_set_error(const char* fmt, ...);
 
 #define MF_LAUNCH_CHECK() MF_CUDA(cudaGetLastError())
 
+// ---------------------------------------------------------------------------------------------
+// Programmatic dependent launch (PDL).  mf_launch() issues a kernel with programmatic stream serialization (unless
+// mf_set_pdl(0) or MF_NO_PDL=1 in the environment): its CTAs may be scheduled, and run their prologue, as soon as every CTA
+// of the kernel before it in the stream has executed mf_pdl_trigger() or exited.  mf_pdl_wait() then blocks until that
+// kernel has completed and its memory operations are visible.  Both instructions are no-ops in a kernel launched without
+// the attribute, so the same kernels serve <<<>>> launches and stream capture unchanged.
+//
+// Hazard rule: mf_pdl_wait() orders a grid only against its IMMEDIATE predecessor.  A kernel launched through mf_launch()
+// therefore touches no global memory (neither reads nor writes) before its mf_pdl_wait(), and every one of them executes it
+// first thing.  Then each such kernel completes only after its predecessor has completed, completion is ordered
+// transitively along the stream, and a buffer written two or more kernels back (the weight image from mlp_prepare, the
+// forward's tile counter pair, the backward's active count, the gradients Adam zeroed) is complete when the wait returns.
+// Moving work that reads such a buffer in front of the wait would be a race: the field kernels also run directly after
+// mf_mlp_prepare (sync_to_module), and the predecessor's own trigger may precede its writes.  (Moving the TMEM / mbarrier
+// set-up of the field kernels in front of the wait was tried: it added spills to the forward kernel.)
+// mf_pdl_trigger() only lets the next grid's CTAs be scheduled; the small kernels issue it right after their wait (their
+// grids fit on the GPU in one wave), the persistent 1-CTA/SM field kernels after the CTA's last tile.
+// Event records between two kernels (mapper.timing, mf_debug_kernel_timer) end the overlap; results are unaffected.
+// ---------------------------------------------------------------------------------------------
+bool mf_pdl_enabled();
+
+template <typename... KArgs, typename... Args>
+static inline cudaError_t mf_launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
+    cfg.attrs = attr; cfg.numAttrs = mf_pdl_enabled() ? 1 : 0;
+    return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
+}
+
+__device__ __forceinline__ void mf_pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void mf_pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
 int mf_sm_count_cached();
 constexpr int MF_KTIMER_SLOTS = 4;
 void mf_ktimer_begin(int slot, cudaStream_t st);   // no-ops unless mf_debug_kernel_timer(1)

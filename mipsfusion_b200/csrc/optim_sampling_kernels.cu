@@ -199,6 +199,7 @@ MF_API int mf_adam_step_sharded(const uint64_t* peer_bases, int world, int rank,
 struct AdamTensor { float4 *p, *g, *m, *v; int64_t n4; AdamScalars a; };
 
 __global__ void __launch_bounds__(256) adam_pair_kernel(AdamTensor t0, AdamTensor t1, int b0) {
+    mf_pdl_wait(); mf_pdl_trigger();
     const bool first = (int)blockIdx.x < b0;
     const AdamTensor& t = first ? t0 : t1;
     const int64_t nb = first ? b0 : (int)gridDim.x - b0, bi = first ? blockIdx.x : blockIdx.x - b0;
@@ -231,8 +232,7 @@ MF_API int mf_adam_step_pair(float* p0, float* g0, float* m0, float* v0, int64_t
     const int64_t cap = (int64_t)mf_sm_count_cached() * 8;
     const int64_t w0 = (t0.n4 + 255) / 256, w1 = (t1.n4 + 255) / 256;
     const int b0 = (int)(w0 < cap ? w0 : cap), b1 = (int)(w1 < 64 ? w1 : 64);
-    adam_pair_kernel<<<(unsigned)(b0 + b1), 256, 0, (cudaStream_t)stream>>>(t0, t1, b0);
-    MF_LAUNCH_CHECK();
+    MF_CUDA(mf_launch(adam_pair_kernel, (unsigned)(b0 + b1), 256, 0, (cudaStream_t)stream, t0, t1, b0));
     return MF_OK;
 }
 

@@ -41,6 +41,7 @@ __global__ void sample_z_kernel(const float* __restrict__ target_d, const float*
                                 unsigned long long* __restrict__ counts, int64_t R) {
     extern __shared__ float zs[];
     __shared__ int cnt[2];
+    mf_pdl_wait(); mf_pdl_trigger();
     const int64_t r = blockIdx.x;
     const int S = c.n_u + c.n_r;
     const bool has_d = target_d != nullptr;
@@ -138,6 +139,7 @@ __global__ void __launch_bounds__(256) render_loss_fwd_kernel(
     const float* __restrict__ target_d, RenderCfgDev c, float* __restrict__ out_rgb, float* __restrict__ out_depth,
     float* __restrict__ out_aux, float* __restrict__ out_w, int32_t* __restrict__ inds, float* __restrict__ scratch,
     int64_t R, int S) {
+    mf_pdl_wait(); mf_pdl_trigger();
     const int64_t r = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (r >= R) return;
@@ -223,6 +225,7 @@ __global__ void __launch_bounds__(1024) loss_finalize_kernel(const float* __rest
                                                              const unsigned long long* __restrict__ counts,
                                                              RenderCfgDev c, float* __restrict__ losses, int64_t R, int S) {
     __shared__ double red[32][8];
+    mf_pdl_wait(); mf_pdl_trigger();
     double s[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     const float4* rows = reinterpret_cast<const float4*>(scratch);            // 8 floats per ray: two 16-byte loads
     for (int64_t r = threadIdx.x; r < R; r += 1024) {
@@ -266,6 +269,7 @@ __global__ void __launch_bounds__(256) render_loss_bwd_kernel(
     const float* __restrict__ target_d, const float* __restrict__ losses, RenderCfgDev c,
     LossGrads g_losses, const float* __restrict__ g_rgb, const float* __restrict__ g_depth,
     float* __restrict__ d_raw, int64_t R, int S) {
+    mf_pdl_wait(); mf_pdl_trigger();
     const int64_t r = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
     if (r >= R) return;
@@ -436,9 +440,8 @@ MF_API int mf_sample_z_ld(const float* target_d, int ld_d, const float* u, const
     cudaStream_t st = (cudaStream_t)stream;
     if (counts) MF_CUDA(cudaMemsetAsync(counts, 0, 2 * sizeof(int64_t), st));
     const int threads = S <= 32 ? 32 : (S <= 64 ? 64 : 128);
-    sample_z_kernel<<<(unsigned)R, threads, S * sizeof(float), st>>>(target_d, u, lin_uniform, lin_range, lin_fallback, c, z,
-                                                                      (unsigned long long*)counts, R);
-    MF_LAUNCH_CHECK();
+    MF_CUDA(mf_launch(sample_z_kernel, (unsigned)R, threads, S * sizeof(float), st, target_d, u, lin_uniform, lin_range, lin_fallback, c, z,
+                      (unsigned long long*)counts, R));
     return MF_OK;
 }
 
@@ -461,13 +464,9 @@ MF_API int mf_render_loss_fwd_ld(const float* raw, const float* z, const float* 
     RenderCfgDev c = cfg_to_dev(cfg);
     c.ld_rgb = ld_rgb; c.ld_d = ld_d;
     cudaStream_t st = (cudaStream_t)stream;
-    render_loss_fwd_kernel<<<(unsigned)((R + 7) / 8), 256, 0, st>>>(raw, z, target_rgb, target_d, c, out_rgb, out_depth, out_aux,
-                                                                   out_weights, inds, scratch, R, S);
-    MF_LAUNCH_CHECK();
-    if (target_d) {
-        loss_finalize_kernel<<<1, 1024, 0, st>>>(scratch, (const unsigned long long*)counts, c, losses, R, S);
-        MF_LAUNCH_CHECK();
-    }
+    MF_CUDA(mf_launch(render_loss_fwd_kernel, (unsigned)((R + 7) / 8), 256, 0, st, raw, z, target_rgb, target_d, c, out_rgb, out_depth, out_aux,
+                      out_weights, inds, scratch, R, S));
+    if (target_d) MF_CUDA(mf_launch(loss_finalize_kernel, 1, 1024, 0, st, scratch, (const unsigned long long*)counts, c, losses, R, S));
     return MF_OK;
 }
 
@@ -482,9 +481,8 @@ static int render_loss_bwd_launch(const float* raw, const float* z, const float*
     if (R == 0) return MF_OK;
     RenderCfgDev c = cfg_to_dev(cfg);
     c.ld_rgb = ld_rgb; c.ld_d = ld_d;
-    render_loss_bwd_kernel<<<(unsigned)((R + 7) / 8), 256, 0, (cudaStream_t)stream>>>(raw, z, target_rgb, target_d, losses, c, gl, g_rgb,
-                                                                                     g_depth, d_raw, R, S);
-    MF_LAUNCH_CHECK();
+    MF_CUDA(mf_launch(render_loss_bwd_kernel, (unsigned)((R + 7) / 8), 256, 0, (cudaStream_t)stream, raw, z, target_rgb, target_d, losses, c,
+                      gl, g_rgb, g_depth, d_raw, R, S));
     return MF_OK;
 }
 
