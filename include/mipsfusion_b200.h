@@ -94,6 +94,21 @@ int mf_set_sm_reserve(int n);
  * stream order.  Process-wide; results are identical either way (A/B switch). */
 int mf_set_pdl(int on);
 int mf_get_pdl(void);
+/* Deterministic mode: 1 = the hash-grid gradient (fixed-point accumulation, independent of point order and timing) and the
+ * pose gradients of gen_rays are bitwise reproducible; 0 = float atomics (default unless MF_DETERMINISTIC=1 in the
+ * environment).  Process-wide.  Where mf_set_bwd_impl(3) would run the four-role tensor-core backward (a feature cache is
+ * given), the call is refused in this mode. */
+int mf_set_deterministic(int on);
+int mf_get_deterministic(void);
+/* Bytes held by the deterministic mode's library-owned workspaces, and their release.  Every (device, stream) that runs a
+ * parameter backward in this mode keeps its own workspace (133.5 MB at 4096 rays x 43 samples, T = 2^19: 144 B per point and
+ * 12 B per grid parameter) until mf_det_release.  A workspace grows only outside stream capture (growth needed under capture
+ * is an error); buffers a larger call outgrows are kept, not freed, so that a CUDA graph captured in this mode stays valid.
+ * mf_det_release synchronises the devices that own one and frees everything: graphs captured in this mode must not be
+ * replayed after it.  Such a graph uses the capturing stream's workspace: do not replay it concurrently with itself or with
+ * deterministic work on that stream. */
+int64_t mf_det_workspace_bytes(void);
+int mf_det_release(void);
 int mf_tc_check_error(void);
 /* Diagnostics: out (128,128) = x (128,K) w (128,K)^T through one tcgen05 layer; K % 16 == 0, K <= 128;
  * passes = 1 (bf16) or 3 (bf16x3 split). */

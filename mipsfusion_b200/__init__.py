@@ -6,6 +6,7 @@ hot path behind the reference's Python call surface.
 The compute lives in ``libmipsfusion_b200.so`` (C ABI, include/mipsfusion_b200.h); importing this
 package does not load it, the first kernel call does -- and raises if it has not been built."""
 from ._lib import MipsFusionB200Error, lib, load_library  # noqa: F401
+from ._lib import set_deterministic, get_deterministic  # noqa: F401
 from .encodings import get_encoder, HashGridEncoding, FrequencyEncoding, IdentityEncoding  # noqa: F401
 from .decoder import MLP_reg  # noqa: F401
 from .scene_rep import JointEncoding  # noqa: F401

@@ -60,6 +60,10 @@ PROTOTYPES = {
     "mf_set_sm_reserve": (_I, [_I]),
     "mf_set_pdl": (_I, [_I]),
     "mf_get_pdl": (_I, []),
+    "mf_set_deterministic": (_I, [_I]),
+    "mf_get_deterministic": (_I, []),
+    "mf_det_workspace_bytes": (_L, []),
+    "mf_det_release": (_I, []),
     "mf_containment": (_I, [_P, _P, _P, _P, _P, _P, _I, _L, _I, _P, _P, _P]),
     "mf_tc_check_error": (_I, []),
     "mf_debug_umma_linear": (_I, [_P, _P, _P, _I, _I, _P]),
@@ -195,3 +199,16 @@ def f32c(t, device=None):
 
 def call(name, *args):
     check(getattr(lib(), name)(*args), name)
+
+
+def set_deterministic(on=True):
+    """Deterministic mode (process-wide, default off unless MF_DETERMINISTIC=1): the hash-grid gradient is formed by fixed-point
+    accumulation and the pose gradients without atomics, so that mapping, bundle adjustment, tracking and the drop-in autograd
+    route give bitwise-identical results on the same inputs, build, GPU model and SM count (DESIGN §4).  Where
+    mf_set_bwd_impl(3) would run the four-role tensor-core backward, the call is refused while it is on.  Each stream used in
+    this mode keeps a library-owned workspace until mf_det_release (see the header)."""
+    call("mf_set_deterministic", 1 if on else 0)
+
+
+def get_deterministic():
+    return bool(lib().mf_get_deterministic())

@@ -194,12 +194,20 @@ __device__ __forceinline__ void encode_backward_tile(const FieldDev& f, const Sr
     if (valid) src.point(i, f, x);
     float dx[3] = {0.f, 0.f, 0.f};
     const float2* grid2 = reinterpret_cast<const float2*>(f.grid);
+    constexpr bool det = is_det_rows<Src>::value;      // grad_grid is the row buffer (mf_common.cuh)
     if (valid) {
 #pragma unroll
         for (int ll = 0; ll < 4; ++ll) {
             const int l = q * 4 + ll;
             const float2 dy = make_float2(G[(2 * l) * LDA + m], G[(2 * l + 1) * LDA + m]);
-            grid_level_bwd<WANT_DX, PARAMS>(x, dy, grid2, grad_grid, level_info(f, l), dx);
+            grid_level_bwd<WANT_DX, PARAMS && !det>(x, dy, grid2, grad_grid, level_info(f, l), dx);
+        }
+        if constexpr (det && PARAMS) {
+            float dy8[8];
+#pragma unroll
+            for (int j = 0; j < 8; ++j) dy8[j] = G[(8 * q + j) * LDA + m];
+            det_store_dy8(grad_grid, slot, q, dy8);
+            if (q == 0) det_store_x(grad_grid, slot, x);
         }
     }
     if (WANT_DX) {

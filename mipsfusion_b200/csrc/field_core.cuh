@@ -54,6 +54,31 @@ struct SrcRays {                         // pts = rays_o + rays_d * z   (model/s
     }
 };
 
+// Point source of the deterministic backward instantiations (mf_common.cuh): the same points, but the kernel writes the
+// grid-gradient rows to grad_grid (the row buffer) instead of scattering.  A distinct type rather than a kernel parameter, so
+// that the default instantiations keep their code and registers.
+template <class S> struct DetRows : S {};
+template <class S> struct is_det_rows { static constexpr bool value = false; };
+template <class S> struct is_det_rows<DetRows<S>> { static constexpr bool value = true; };
+
+__device__ __forceinline__ void det_store_x(float* rows, int64_t slot, const float x[3]) {
+    *reinterpret_cast<float4*>(rows + slot * MF_DET_ROW) = make_float4(x[0], x[1], x[2], 0.f);
+}
+// the whole row: x and the 32 gradient words (role-split backward, field_tc_bwd2.cuh)
+__device__ __forceinline__ void det_store_row(float* rows, int64_t slot, const float x[3], const uint32_t (&r)[32]) {
+    float4* row = reinterpret_cast<float4*>(rows + slot * MF_DET_ROW);
+    row[0] = make_float4(x[0], x[1], x[2], 0.f);
+#pragma unroll
+    for (int j = 0; j < 8; ++j)
+        row[1 + j] = make_float4(__uint_as_float(r[4 * j]), __uint_as_float(r[4 * j + 1]), __uint_as_float(r[4 * j + 2]), __uint_as_float(r[4 * j + 3]));
+}
+// the gradients of levels 4 q .. 4 q + 3
+__device__ __forceinline__ void det_store_dy8(float* rows, int64_t slot, int q, const float dy[8]) {
+    float4* r = reinterpret_cast<float4*>(rows + slot * MF_DET_ROW + MF_DET_DY + 8 * q);
+    r[0] = make_float4(dy[0], dy[1], dy[2], dy[3]);
+    r[1] = make_float4(dy[4], dy[5], dy[6], dy[7]);
+}
+
 // ------------------------------------------------------------------------------------------
 // Encode one tile: thread (m = tid & 63, q = tid >> 6) handles 4 grid levels and 12 frequency
 // outputs of point m.

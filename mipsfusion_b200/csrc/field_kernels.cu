@@ -287,23 +287,7 @@ __global__ void hashgrid_fwd_kernel(FieldDev f, const float* __restrict__ x, flo
 template <bool WANT_DX>
 __global__ void hashgrid_bwd_kernel(FieldDev f, const float* __restrict__ x, const float* __restrict__ dy,
                                     float* __restrict__ grad, float* __restrict__ dx_out, int64_t N) {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int L = f.n_levels;                       // 16 levels -> the 16 lanes of a half warp share a point
-    const bool active = t < N * L;
-    const int64_t i = active ? t / L : 0; const int l = (int)(t % L);
-    float dx[3] = {0.f, 0.f, 0.f};
-    if (active) {
-        const float xv[3] = {x[i * 3], x[i * 3 + 1], x[i * 3 + 2]};
-        const float2 g = reinterpret_cast<const float2*>(dy)[t];
-        grid_level_bwd<WANT_DX>(xv, g, reinterpret_cast<const float2*>(f.grid), grad, level_info(f, l), dx);
-    }
-    if (WANT_DX) {
-#pragma unroll
-        for (int d = 0; d < 3; ++d)
-#pragma unroll
-            for (int o = 8; o > 0; o >>= 1) dx[d] += __shfl_xor_sync(0xffffffffu, dx[d], o);
-        if (active && l == 0) { dx_out[i * 3] = dx[0]; dx_out[i * 3 + 1] = dx[1]; dx_out[i * 3 + 2] = dx[2]; }
-    }
+    hashgrid_bwd_body<WANT_DX, true>(f, x, dy, grad, dx_out, N);
 }
 
 __global__ void freq_fwd_kernel(const float* __restrict__ x, float* __restrict__ out, int D, int K, int64_t N) {
@@ -366,6 +350,11 @@ static int meta_to_dev(const mf_grid_meta* m, const float* grid, FieldDev* d) {
     return MF_OK;
 }
 
+// floats of the table (the gradient's length)
+static inline int64_t det_params(const FieldDev& d) {
+    return 2 * ((int64_t)d.offset[d.n_levels - 1] + d.size[d.n_levels - 1]);
+}
+
 MF_API int mf_hashgrid_meta(int log2_T, int n_levels, int n_features, int base_res, double per_level_scale, mf_grid_meta* m) {
     MF_CHECK_ARG(m != nullptr);
     MF_CHECK_ARG(n_levels >= 1 && n_levels <= MF_MAX_LEVELS);
@@ -418,6 +407,15 @@ MF_API int mf_hashgrid_bwd(const float* x, const float* dL_dy, const float* grid
     if (dL_dx && d.n_levels != 16) { mf_set_error("mf_hashgrid_bwd: input gradient needs 16 levels"); return MF_ERR_UNSUPPORTED; }
     const int64_t T = N * d.n_levels;
     const unsigned blocks = (unsigned)((T + 255) / 256);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (mf_deterministic()) {
+        if (dL_dx) {
+            rc = mf_det_hashgrid_dx(d, x, dL_dy, dL_dx, N, st); if (rc) return rc;
+        }
+        DetWs ws;
+        rc = mf_det_workspace(0, det_params(d), st, &ws); if (rc) return rc;
+        return mf_det_scatter(d, ws, x, 3, dL_dy, 2 * d.n_levels, nullptr, N, grad_grid, st);
+    }
     if (dL_dx) hashgrid_bwd_kernel<true><<<blocks, 256, 0, (cudaStream_t)stream>>>(d, x, dL_dy, grad_grid, dL_dx, N);
     else hashgrid_bwd_kernel<false><<<blocks, 256, 0, (cudaStream_t)stream>>>(d, x, dL_dy, grad_grid, nullptr, N);
     MF_LAUNCH_CHECK();
@@ -574,42 +572,44 @@ MF_API int64_t mf_field_bwd_workspace_size(int64_t n_points, int want_point_grad
     return mf_mlp_grad_workspace_size() + (want_point_grads ? 3 * n_points : 0) + act_scratch_words(n_points) + cta_scratch_words();
 }
 
+// The kernels of one backward after the compaction.  With Src = DetRows<...> (deterministic mode) grad_grid is the row buffer.
 template <class Src>
-static int launch_field_bwd(const FieldDev& d, const Src& src, const float* d_raw, float* grad_grid, float* grad_mlp,
-                            float* d_pts, float* workspace, float* scratch, int64_t N, cudaStream_t st) {
-    // workspace: per-CTA partials; scratch: act_scratch_words(N) words for the active-point list
-    ActiveMap am{nullptr, nullptr};
-    int rc0 = compact_active_points(d_raw, N, scratch, &am, st); if (rc0) return rc0;
-    if (d_pts) MF_CUDA(cudaMemsetAsync(d_pts, 0, (size_t)N * 3 * sizeof(float), st));   // skipped points: exactly zero
+static int launch_field_bwd_kernels(const FieldDev& d, const Src& src, const float* d_raw, float* grad_grid, float* grad_mlp,
+                                    float* d_pts, float* workspace, float* scratch, int64_t N, const ActiveMap& am, cudaStream_t st) {
+    constexpr bool det = is_det_rows<Src>::value;
     const bool params = grad_grid != nullptr;          // false: input gradients only (pose refinement, overlap consistency)
-    if (!params && !d_pts) {
-        mf_set_error("backward without parameter gradients needs a ray / point gradient output");
-        return MF_ERR_INVALID;
-    }
-    if (!params && d.impl == 1) {
-        const int grid = persistent_grid(N, 1);
-        int rc = set_smem(field_bwd_dx_kernel<Src>, SMEM_BWD); if (rc) return rc;
-        field_bwd_dx_kernel<Src><<<grid, NT, SMEM_BWD, st>>>(d, src, d_raw, d_pts, N, am);
-        MF_LAUNCH_CHECK();
-        return MF_OK;
+    if constexpr (!det) {
+        if (!params && d.impl == 1) {
+            const int grid = persistent_grid(N, 1);
+            int rc = set_smem(field_bwd_dx_kernel<Src>, SMEM_BWD); if (rc) return rc;
+            field_bwd_dx_kernel<Src><<<grid, NT, SMEM_BWD, st>>>(d, src, d_raw, d_pts, N, am);
+            MF_LAUNCH_CHECK();
+            return MF_OK;
+        }
     }
     if (d.impl != 1) {                                 // tcgen05 path: 128-point tiles, one CTA per SM
         const int64_t tiles = (N + TC_TP - 1) / TC_TP;
         const int64_t cap = mf_sm_count_cached();
         const int grid = (int)(tiles < cap ? (tiles > 0 ? tiles : 1) : cap);
         mf_ktimer_begin(1, st);
-        if (!params) {
-            int rc = set_smem(field_bwd_tc_kernel<Src, true, false>, SMEM_TC_BWD); if (rc) return rc;
-            field_bwd_tc_kernel<Src, true, false><<<grid, TC_NT, SMEM_TC_BWD, st>>>(d, src, d_raw, nullptr, nullptr, d_pts, N, am, mf_tc_error_flag(), mf_tc_profile_buffer());
-            mf_ktimer_end(1, st);
-            MF_LAUNCH_CHECK();
-            return MF_OK;
+        if constexpr (!det) {
+            if (!params) {
+                int rc = set_smem(field_bwd_tc_kernel<Src, true, false>, SMEM_TC_BWD); if (rc) return rc;
+                field_bwd_tc_kernel<Src, true, false><<<grid, TC_NT, SMEM_TC_BWD, st>>>(d, src, d_raw, nullptr, nullptr, d_pts, N, am, mf_tc_error_flag(), mf_tc_profile_buffer());
+                mf_ktimer_end(1, st);
+                MF_LAUNCH_CHECK();
+                return MF_OK;
+            }
         }
-        if (!d_pts && mf_bwd_impl() != 1) {                // role-split kernels (parameter gradients only)
+        if (!d_pts && (det || mf_bwd_impl() != 1)) {       // role-split kernels (parameter gradients only)
             uint32_t* cta_scr = reinterpret_cast<uint32_t*>(scratch + act_scratch_words(N));
-            if (mf_bwd_impl() == 3 && d.feat) {            // four roles (A/B only: measured slower, field_tc_bwd3.cuh); needs the feature cache
-                int rc = set_smem(field_bwd_tc3_kernel<Src>, b3::SMEM); if (rc) return rc;
-                field_bwd_tc3_kernel<Src><<<grid, b3::B3_NT, b3::SMEM, st>>>(d, src, d_raw, grad_grid, workspace, cta_scr, N, am, mf_tc_error_flag(), mf_tc_profile_buffer());
+            bool four_roles = false;
+            if constexpr (!det) four_roles = mf_bwd_impl() == 3 && d.feat != nullptr;
+            if (four_roles) {                              // four roles (A/B only: measured slower, field_tc_bwd3.cuh); needs the feature cache
+                if constexpr (!det) {
+                    int rc = set_smem(field_bwd_tc3_kernel<Src>, b3::SMEM); if (rc) return rc;
+                    field_bwd_tc3_kernel<Src><<<grid, b3::B3_NT, b3::SMEM, st>>>(d, src, d_raw, grad_grid, workspace, cta_scr, N, am, mf_tc_error_flag(), mf_tc_profile_buffer());
+                }
             } else {                                       // three roles (default)
                 int rc = set_smem(field_bwd_tc2_kernel<Src>, b2::SMEM); if (rc) return rc;
                 MF_CUDA(mf_launch(field_bwd_tc2_kernel<Src>, grid, b2::B2_NT, b2::SMEM, st, d, src, d_raw, grad_grid, workspace, cta_scr, N, am,
@@ -620,17 +620,19 @@ static int launch_field_bwd(const FieldDev& d, const Src& src, const float* d_ra
             MF_CUDA(mf_launch(reduce_partials_kernel, (MF_MLP_PARAMS + 31) / 32 + 1, 256, 0, st, workspace, grid, grad_mlp, 2, d.prep));
             return MF_OK;
         }
-        if (d_pts) {
-            int rc = set_smem(field_bwd_tc_kernel<Src, true>, SMEM_TC_BWD); if (rc) return rc;
-            field_bwd_tc_kernel<Src, true><<<grid, TC_NT, SMEM_TC_BWD, st>>>(d, src, d_raw, grad_grid, workspace, d_pts, N, am, mf_tc_error_flag(), mf_tc_profile_buffer());
-        } else {
-            int rc = set_smem(field_bwd_tc_kernel<Src, false>, SMEM_TC_BWD); if (rc) return rc;
-            field_bwd_tc_kernel<Src, false><<<grid, TC_NT, SMEM_TC_BWD, st>>>(d, src, d_raw, grad_grid, workspace, nullptr, N, am, mf_tc_error_flag(), mf_tc_profile_buffer());
+        if constexpr (!det) {                           // (deterministic mode: launch_field_bwd never gets here)
+            if (d_pts) {
+                int rc = set_smem(field_bwd_tc_kernel<Src, true>, SMEM_TC_BWD); if (rc) return rc;
+                field_bwd_tc_kernel<Src, true><<<grid, TC_NT, SMEM_TC_BWD, st>>>(d, src, d_raw, grad_grid, workspace, d_pts, N, am, mf_tc_error_flag(), mf_tc_profile_buffer());
+            } else {
+                int rc = set_smem(field_bwd_tc_kernel<Src, false>, SMEM_TC_BWD); if (rc) return rc;
+                field_bwd_tc_kernel<Src, false><<<grid, TC_NT, SMEM_TC_BWD, st>>>(d, src, d_raw, grad_grid, workspace, nullptr, N, am, mf_tc_error_flag(), mf_tc_profile_buffer());
+            }
+            mf_ktimer_end(1, st);
+            MF_LAUNCH_CHECK();
+            reduce_partials_kernel<<<(MF_MLP_PARAMS + 31) / 32, 256, 0, st>>>(workspace, grid, grad_mlp, 1, nullptr);
+            MF_LAUNCH_CHECK();
         }
-        mf_ktimer_end(1, st);
-        MF_LAUNCH_CHECK();
-        reduce_partials_kernel<<<(MF_MLP_PARAMS + 31) / 32, 256, 0, st>>>(workspace, grid, grad_mlp, 1, nullptr);
-        MF_LAUNCH_CHECK();
         return MF_OK;
     }
     const int grid = persistent_grid(N, 1);
@@ -645,6 +647,37 @@ static int launch_field_bwd(const FieldDev& d, const Src& src, const float* d_ra
     reduce_partials_kernel<<<(MF_MLP_PARAMS + 31) / 32, 256, 0, st>>>(workspace, grid, grad_mlp, 0, nullptr);
     MF_LAUNCH_CHECK();
     return MF_OK;
+}
+
+template <class Src>
+static int launch_field_bwd(const FieldDev& d, const Src& src, const float* d_raw, float* grad_grid, float* grad_mlp,
+                            float* d_pts, float* workspace, float* scratch, int64_t N, cudaStream_t st) {
+    // workspace: per-CTA partials; scratch: act_scratch_words(N) words for the active-point list
+    const bool params = grad_grid != nullptr;
+    if (!params && !d_pts) {
+        mf_set_error("backward without parameter gradients needs a ray / point gradient output");
+        return MF_ERR_INVALID;
+    }
+    const bool det = params && mf_deterministic();
+    if (det && d.impl != 1 && !d_pts && mf_bwd_impl() == 3 && d.feat) {     // (where the default mode runs the four-role kernel)
+        mf_set_error("deterministic mode: the four-role tensor-core backward (mf_set_bwd_impl(3)) scatters with float atomics and is "
+                     "not available; select another backward");
+        return MF_ERR_UNSUPPORTED;
+    }
+    DetWs ws{};
+    if (det) { int rc = mf_det_workspace(N, det_params(d), st, &ws); if (rc) return rc; }
+    ActiveMap am{nullptr, nullptr};
+    int rc0 = compact_active_points(d_raw, N, scratch, &am, st); if (rc0) return rc0;
+    if (d_pts) MF_CUDA(cudaMemsetAsync(d_pts, 0, (size_t)N * 3 * sizeof(float), st));   // skipped points: exactly zero
+    if (!det) return launch_field_bwd_kernels(d, src, d_raw, grad_grid, grad_mlp, d_pts, workspace, scratch, N, am, st);
+    // Tensor cores with point gradients: the single-role kernel sums its decoder partials from four warps in no fixed order, so
+    // the input gradients come from its PARAMS = false instantiation and the parameter gradients from the role-split kernel.
+    const bool split = d.impl != 1 && d_pts;
+    if (split) { int rc = launch_field_bwd_kernels(d, src, d_raw, nullptr, nullptr, d_pts, workspace, scratch, N, am, st); if (rc) return rc; }
+    // rows of the active slots [0, count), then the fixed-point passes over them
+    int rc = launch_field_bwd_kernels(d, DetRows<Src>{src}, d_raw, ws.rows, grad_mlp, split ? nullptr : d_pts, workspace, scratch, N, am, st);
+    if (rc) return rc;
+    return mf_det_scatter(d, ws, ws.rows, MF_DET_ROW, ws.rows + MF_DET_DY, MF_DET_ROW, am.count, N, grad_grid, st);
 }
 
 MF_API int mf_field_query(const float* pts, const mf_field* field, int normalize, float* out, int64_t N, void* stream) {

@@ -740,7 +740,7 @@ __global__ void __launch_bounds__(b2::B2_NT, 1) field_bwd_tc2_kernel(FieldDev f,
             // use the unit just as much)
             if (prof && blockIdx.x == 0 && k == 1 && p == 0) prof[26] = clock64();
 #ifndef MF_EXP_NOSCATTER
-            {
+            if constexpr (is_det_rows<Src>::value) { if (valid) det_store_row(grad_grid, slot, x, r); } else {   // (deterministic mode)
                 // (slots behind the end of the list carry an all-zero gradient row: they join the runs with zeros and are skipped)
 #pragma unroll 1
                 for (int gq = 0; gq < 4; ++gq) {         // rolled over groups of 4 levels: three roles share the instruction cache

@@ -164,6 +164,29 @@ __device__ __forceinline__ void grid_level_bwd(const float x[3], float2 dy, cons
     }
 }
 
+// Backward of the stand-alone encoding (mf_hashgrid_bwd): thread per (point, level).
+template <bool WANT_DX, bool SCATTER>
+__device__ __forceinline__ void hashgrid_bwd_body(const FieldDev& f, const float* __restrict__ x, const float* __restrict__ dy,
+                                                  float* __restrict__ grad, float* __restrict__ dx_out, int64_t N) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int L = f.n_levels;                       // 16 levels -> the 16 lanes of a half warp share a point
+    const bool active = t < N * L;
+    const int64_t i = active ? t / L : 0; const int l = (int)(t % L);
+    float dx[3] = {0.f, 0.f, 0.f};
+    if (active) {
+        const float xv[3] = {x[i * 3], x[i * 3 + 1], x[i * 3 + 2]};
+        const float2 g = reinterpret_cast<const float2*>(dy)[t];
+        grid_level_bwd<WANT_DX, SCATTER>(xv, g, reinterpret_cast<const float2*>(f.grid), grad, level_info(f, l), dx);
+    }
+    if (WANT_DX) {
+#pragma unroll
+        for (int d = 0; d < 3; ++d)
+#pragma unroll
+            for (int o = 8; o > 0; o >>= 1) dx[d] += __shfl_xor_sync(0xffffffffu, dx[d], o);
+        if (active && l == 0) { dx_out[i * 3] = dx[0]; dx_out[i * 3 + 1] = dx[1]; dx_out[i * 3 + 2] = dx[2]; }
+    }
+}
+
 // Warp-aggregated scatter of one level (all 32 lanes of the warp call it together; lane = point, consecutive lanes = consecutive
 // active points = mostly consecutive samples of one ray).  Consecutive samples share their cell on the coarse levels -- the samples
 // a loss term sees sit within the truncation distance of the surface, a few centimetres apart -- so lanes are grouped into runs of

@@ -105,6 +105,21 @@ MF_API int mf_set_pdl(int on) {
 }
 MF_API int mf_get_pdl(void) { return mf_pdl_enabled() ? 1 : 0; }
 
+// Deterministic mode (det_kernels.cu): off unless MF_DETERMINISTIC=1; mf_set_deterministic switches it at run time.
+static int g_det = -1;
+bool mf_deterministic() {
+    if (g_det < 0) {
+        const char* e = getenv("MF_DETERMINISTIC");
+        g_det = (e && e[0] && strcmp(e, "0") != 0) ? 1 : 0;
+    }
+    return g_det != 0;
+}
+MF_API int mf_set_deterministic(int on) {
+    g_det = on ? 1 : 0;
+    return MF_OK;
+}
+MF_API int mf_get_deterministic(void) { return mf_deterministic() ? 1 : 0; }
+
 static int* g_tc_err[64] = {nullptr};
 int* mf_tc_error_flag() {
     int dev = 0;

@@ -140,6 +140,31 @@ struct ActiveMap {
     __device__ __forceinline__ int64_t operator()(int64_t slot) const { return idx ? (int64_t)idx[slot] : slot; }
 };
 
+// ---------------------------------------------------------------------------------------------
+// Deterministic mode (mf_set_deterministic, det_kernels.cu).  The backward kernels' deterministic instantiations (point source
+// DetRows<Src>, field_core.cuh) do not scatter into the table: they write one row of MF_DET_ROW floats per active slot -- the
+// normalised position at [0, 3), the 32 grid-feature gradients at [MF_DET_DY, MF_DET_DY + 32) -- and mf_det_scatter forms
+// grad += sum of the contributions by fixed-point accumulation, whose result depends only on the multiset of contributions.
+// ---------------------------------------------------------------------------------------------
+constexpr int MF_DET_ROW = 36;
+constexpr int MF_DET_DY = 4;
+constexpr int MF_DET_MAX_H = 35;      // headroom bits: 8 N + 1 <= 2^35 (N < 2^32 points per launch)
+bool mf_deterministic();
+struct DetWs {
+    float* rows;                      // [n][MF_DET_ROW]
+    uint32_t* expo;                   // [P] per gradient float: max exponent of its contributions | non-finite flags (zero between calls)
+    unsigned long long* acc;          // [P] fixed-point sums (zero between calls)
+};
+// The library-owned workspace of (current device, st) with room for n rows and P gradient floats; grows outside stream
+// capture only (an error under capture).  Outgrown buffers are retired, not freed, until mf_det_release (captured graphs).
+int mf_det_workspace(int64_t n, int64_t P, cudaStream_t st, DetWs* ws);
+// grad[e] += sum of __fmul_rn(w, dy) over the (point, level, corner) contributions to e of the n points (x[i * ldx + d],
+// dy[i * ldy + 2 l + k]); count (device, may be NULL) limits the points to its value.  Three kernels through mf_launch.
+int mf_det_scatter(const FieldDev& f, const DetWs& ws, const float* x, int ldx, const float* dy, int ldy, const int* count, int64_t n,
+                   float* grad, cudaStream_t st);
+// dx (N, 3) of the stand-alone hash-grid encoding (16 levels) without the table scatter
+int mf_det_hashgrid_dx(const FieldDev& f, const float* x, const float* dy, float* dx, int64_t N, cudaStream_t st);
+
 int mf_field_to_dev(const mf_field* f, FieldDev* d);   // validates (16 levels, 2 features)
 int mf_decoder_impl();                                 // 0: tcgen05 tensor cores (default), 1: fp32 CUDA cores
 int mf_bwd_impl();                                     // tensor-core backward: 0 role-split kernel (default), 1 single-role kernel

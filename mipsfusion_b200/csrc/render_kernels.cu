@@ -419,6 +419,50 @@ __global__ void __launch_bounds__(256) gen_rays_bwd_kernel(const float* __restri
     }
 }
 
+// Deterministic mode: the same gradient without atomics.  Block k owns pose k: its threads scan the rays in a fixed strided order,
+// a fixed shared-memory tree combines them, and one thread adds each entry to d_poses.  No workspace: capturable as it is.
+constexpr int GRB_DET_NT = 256;
+__global__ void __launch_bounds__(GRB_DET_NT) gen_rays_bwd_det_kernel(const float* __restrict__ dirs, int dir_stride,
+                                                                      const int64_t* __restrict__ pose_idx, const float* __restrict__ d_o,
+                                                                      const float* __restrict__ d_d, float* __restrict__ d_poses, int64_t R, int K) {
+    __shared__ float red[12][GRB_DET_NT];
+    const int k = blockIdx.x, t = threadIdx.x;
+    float a[12];
+#pragma unroll
+    for (int e = 0; e < 12; ++e) a[e] = 0.f;
+    for (int64_t r = t; r < R; r += GRB_DET_NT) {
+        int64_t pi = pose_idx ? pose_idx[r] : 0;
+        if (pi < 0) pi += K;
+        if (pi != k) continue;
+        const float dv[3] = {dirs[r * dir_stride], dirs[r * dir_stride + 1], dirs[r * dir_stride + 2]};
+#pragma unroll
+        for (int j = 0; j < 3; ++j) {
+            const float g = d_d[r * 3 + j];
+#pragma unroll
+            for (int c = 0; c < 3; ++c) a[j * 4 + c] = __fadd_rn(a[j * 4 + c], __fmul_rn(g, dv[c]));
+            a[j * 4 + 3] = __fadd_rn(a[j * 4 + 3], d_o[r * 3 + j]);
+        }
+    }
+#pragma unroll
+    for (int e = 0; e < 12; ++e) red[e][t] = a[e];
+    __syncthreads();
+    for (int s = GRB_DET_NT / 2; s > 0; s >>= 1) {
+        if (t < s)
+#pragma unroll
+            for (int e = 0; e < 12; ++e) red[e][t] = __fadd_rn(red[e][t], red[e][t + s]);
+        __syncthreads();
+    }
+    if (t < 12) d_poses[(int64_t)k * 16 + t] = __fadd_rn(d_poses[(int64_t)k * 16 + t], red[t][0]);
+}
+
+static int gen_rays_bwd_launch(const float* dirs, int stride, const int64_t* pose_idx, const float* d_o, const float* d_d, float* d_poses,
+                               int64_t R, int K, cudaStream_t st) {
+    if (mf_deterministic()) gen_rays_bwd_det_kernel<<<(unsigned)K, GRB_DET_NT, 0, st>>>(dirs, stride, pose_idx, d_o, d_d, d_poses, R, K);
+    else gen_rays_bwd_kernel<<<(unsigned)((R + 255) / 256), 256, 0, st>>>(dirs, stride, pose_idx, d_o, d_d, d_poses, R, K);
+    MF_LAUNCH_CHECK();
+    return MF_OK;
+}
+
 // ---------------------------------------------------------------------------------------------
 MF_API int mf_sample_z(const float* target_d, const float* u, const float* lin_uniform, const float* lin_range,
                        const float* lin_fallback, const mf_render_cfg* cfg, float* z, int64_t* counts, int64_t R, void* stream) {
@@ -531,9 +575,7 @@ MF_API int mf_gen_rays_bwd(const float* dirs_cam, const int64_t* pose_idx, const
     MF_CHECK_ARG(R >= 0 && K >= 1);
     if (R == 0) return MF_OK;
     MF_CHECK_ARG(dirs_cam && d_rays_o && d_rays_d && d_poses);
-    gen_rays_bwd_kernel<<<(unsigned)((R + 255) / 256), 256, 0, (cudaStream_t)stream>>>(dirs_cam, 3, pose_idx, d_rays_o, d_rays_d, d_poses, R, K);
-    MF_LAUNCH_CHECK();
-    return MF_OK;
+    return gen_rays_bwd_launch(dirs_cam, 3, pose_idx, d_rays_o, d_rays_d, d_poses, R, K, (cudaStream_t)stream);
 }
 
 MF_API int mf_gen_rays_packed_bwd(const float* rays7, const int64_t* pose_idx, const float* d_rays_o, const float* d_rays_d,
@@ -541,7 +583,5 @@ MF_API int mf_gen_rays_packed_bwd(const float* rays7, const int64_t* pose_idx, c
     MF_CHECK_ARG(R >= 0 && K >= 1);
     if (R == 0) return MF_OK;
     MF_CHECK_ARG(rays7 && d_rays_o && d_rays_d && d_poses);
-    gen_rays_bwd_kernel<<<(unsigned)((R + 255) / 256), 256, 0, (cudaStream_t)stream>>>(rays7, 7, pose_idx, d_rays_o, d_rays_d, d_poses, R, K);
-    MF_LAUNCH_CHECK();
-    return MF_OK;
+    return gen_rays_bwd_launch(rays7, 7, pose_idx, d_rays_o, d_rays_d, d_poses, R, K, (cudaStream_t)stream);
 }

@@ -3,7 +3,13 @@ z, counts, raw, rgb, depth, losses, d_raw, the active-point list, the decoder gr
 then the decoder and grid after Adam.  Two builds (or two runs of one build) are compared with scripts/compare_dumps.py; all
 buffers but the grid gradient and the grid (float atomic scatter) are expected to be bitwise equal.
 
-    python scripts/dump_step.py DIR"""
+With --deterministic (mipsfusion_b200.set_deterministic) the grid gradient is order-independent too, and --steps K dumps the
+K-th step (K - 1 full steps with Adam before it, the same draw u every step).  DIR/mode.json records the mode; when both
+directories are deterministic dumps, compare_dumps.py expects EVERY buffer bitwise equal and exits non-zero otherwise.
+
+    python scripts/dump_step.py DIR [--deterministic] [--steps K]"""
+import argparse
+import json
 import os
 import sys
 
@@ -15,8 +21,9 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 
-def main(out):
+def main(out, deterministic=False, steps=1):
     import bench
+    import mipsfusion_b200 as mf
     import helpers as H
     from mipsfusion_b200 import _lib as L
     from mipsfusion_b200.decoder import _Workspace
@@ -34,6 +41,9 @@ def main(out):
     cfg_r, _ = model._render_cfg(True, 0.01, dev)
     S = cfg_r.n_samples_d + cfg_r.n_range_d
     u = torch.rand(R, S, generator=torch.Generator().manual_seed(1234)).to(dev)     # host-seeded draw: the same in every build
+    mf.set_deterministic(deterministic)
+    for _ in range(steps - 1):
+        mapper.step(ro, rd, tc, td, u=u)
     losses = mapper.step(ro, rd, tc, td, u=u, update=False)
     torch.cuda.synchronize()
     b = mapper._buffers(R, S)
@@ -54,8 +64,15 @@ def main(out):
     arrs["grid_after_adam"] = mapper.grid.cpu().numpy().copy()
     for k, v in arrs.items():
         np.save(os.path.join(out, k + ".npy"), v)
-    print("dumped", sorted(arrs), "n_active", arrs["active"].size)
+    with open(os.path.join(out, "mode.json"), "w") as f:
+        json.dump({"deterministic": bool(deterministic), "steps": steps}, f)
+    print("dumped", sorted(arrs), "n_active", arrs["active"].size, "deterministic", bool(deterministic), "steps", steps)
 
 
 if __name__ == "__main__":
-    main(sys.argv[1])
+    ap = argparse.ArgumentParser()
+    ap.add_argument("dir")
+    ap.add_argument("--deterministic", action="store_true")
+    ap.add_argument("--steps", type=int, default=1)
+    a = ap.parse_args()
+    main(a.dir, a.deterministic, max(a.steps, 1))
